@@ -2,9 +2,12 @@
 """bench.py -- throughput of the BreakID hot path on B200 (BASELINE.json metric: read pairs/s classified + clustered
 + refined; decode excluded AND included, both stated).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl reference] [--dump-outputs DIR]
 
-One JSON line.  What the keys mean here:
+One JSON line.  Every throughput below (value, e2e, e2e_host_soa, legs) is measured over exactly K timed steps; the
+per-kernel and per-stage breakdowns come from two extra steps of their own.  With the same arguments the inputs are the
+same from run to run (seeded generators), so DIR (see dump_outputs) lets two builds be compared output for output.
+What the keys mean here:
 
   value     BASELINE.json configs[1] (hg19-shaped 3.1 Gb genome, 30x 2x150 bp, 2000 planted SVs, 1 % chimeric noise;
             --scale shrinks it), records RESIDENT in HBM when the timed region starts, decode EXCLUDED.  A step is one
@@ -274,8 +277,10 @@ def rank_slice(cfg, rank, world, dev):
 # ------------------------------------------------------------------------------------------------------------------
 # the bounded sample both arms share (decode included)
 # ------------------------------------------------------------------------------------------------------------------
-def sample_dataset(scale):
-    """BAM + index + nib + refGene of configs[1] x scale in a per-box cache directory (whichever arm runs first writes it)"""
+def sample_dataset(scale, index=False):
+    """BAM + nib + refGene of configs[1] x scale in a cache directory under the system temporary directory (whichever arm
+    runs first writes it).  index=True adds the .bai index, which only the reference binary reads; it is built with
+    oracle/_ref/bamindex, so only where the reference is built."""
     import oracle_py as O
     from breakid_b200 import bamio
     d = os.path.join(tempfile.gettempdir(), "bkid_sample_1_%d" % round(1 / scale))
@@ -286,9 +291,10 @@ def sample_dataset(scale):
         data = synth.generate(workload_cfg(scale))
         t0 = time.time()
         bamio.write_dataset(d, data, random_qual=True)
-        O.ref_index(paths["bam"])
         with open(done, "w") as f:
             f.write("%d %.1f\n" % (data.n, time.time() - t0))
+    if index and not os.path.exists(paths["bam"] + ".bai"):
+        O.ref_index(paths["bam"])
     n = int(open(done).read().split()[0])
     return paths, n
 
@@ -437,7 +443,7 @@ def exclude_intervals(cfg, frac=0.05, seed=3):
     return np.array(t, np.int32), np.array(b, np.int32), np.array(e, np.int32)
 
 
-def align_leg(local, n_pairs=1 << 20):
+def align_leg(local, steps, n_pairs=1 << 20):
     """north_star kernel 4 (banded alignment; extension, default off): clipped reads of length U(20,130) against their
     reference window, band 12.  pairs/s and cell updates/s of the kernel alone (host arrays in, device timing inside)."""
     rng = np.random.RandomState(5)
@@ -454,7 +460,7 @@ def align_leg(local, n_pairs=1 << 20):
     ts = []
     api.profile_kernels(True)
     api.profile_report()
-    for i in range(4):
+    for i in range(steps):
         t0 = time.perf_counter()
         ctx._chk(ctx.lib.bkid_op_banded_align(ctx.ctx, n_pairs, p(q), p(off), p(r), p(off), 12, p(out)))
         ts.append(time.perf_counter() - t0)
@@ -502,6 +508,32 @@ def kernel_bytes(name, cnt, n):
     if name.startswith("k2_build_pairs"):
         return 4.0 * nc + (2 * 48.0 + 64.0) * npair, "mate 4 per candidate; two rows read + one pair written per pair"
     return None, None
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirpath, res, calls):
+    """what one step of the timed path hands its caller, as float64 arrays: insert_mean, insert_sd, cluster_dist and n_called
+    from bkid_run, and call_<field> for every field of the call records of bkid_fetch_clusters (the 41-mer fields as
+    [n, 44] byte codes).  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the calls is written, and call_index
+    holds their positions."""
+    os.makedirs(dirpath, exist_ok=True)
+    arrays = {k: np.array([v], np.float64) for k, v in zip(("insert_mean", "insert_sd", "cluster_dist", "n_called"), res)}
+    fields = {}
+    for k in calls.dtype.names:
+        a = np.ascontiguousarray(calls[k])
+        fields["call_" + k] = a.view(np.uint8).reshape(len(a), a.dtype.itemsize) if a.dtype.kind == "S" else a
+    row_bytes = 8 * (1 + sum(dt.itemsize if dt.kind == "S" else 1 for dt, _ in calls.dtype.fields.values()))     # + call_index
+    keep = (DUMP_LIMIT_BYTES - (1 << 16)) // row_bytes          # 64 KiB left for the scalars and the .npy headers
+    if len(calls) > keep:
+        idx = np.sort(np.random.RandomState(0).choice(len(calls), keep, replace=False))
+        fields = {k: a[idx] for k, a in fields.items()}
+        arrays["call_index"] = idx.astype(np.float64)
+    for k, a in fields.items():
+        arrays[k] = a.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirpath, k + ".npy"), a)
 
 
 def run_ours(args):
@@ -603,7 +635,10 @@ def run_ours(args):
     ncall = res[3]
     deterministic = None
     if world == 1:
-        deterministic = bool(ctx.fetch_clusters().tobytes() == ref_out.tobytes())
+        last_out = ctx.fetch_clusters()
+        deterministic = bool(last_out.tobytes() == ref_out.tobytes())
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res, last_out)
     # ---- N > 1: per-stage / per-collective wall times of the sharded step (extra untimed steps with a sync after every stage) ----
     if world > 1:
         timing_on[0] = True
@@ -639,11 +674,10 @@ def run_ours(args):
         step_e2e()
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(args.steps, 3))
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         r, out = step_e2e()
     barrier()
-    soa_ms = (time.perf_counter() - t0) * 1e3 / e2e_steps
+    soa_ms = (time.perf_counter() - t0) * 1e3 / args.steps
     d2h_bytes = int(out.nbytes) if out is not None else 192 * int(r[3])
 
     # max over ranks
@@ -726,7 +760,7 @@ def run_ours(args):
     # ---- e2e: decode included, on the file the reference arm runs on ----
     s_scale = min(sample_scale(args.steps, args.warmup), args.scale)
     if world > 1 and not args.no_decode:
-        e = decode_included_sharded(rank, world, local, dev, max(1, min(args.steps, 10)), 2, s_scale)
+        e = decode_included_sharded(rank, world, local, dev, args.steps, 2, s_scale)
         if rank == 0:
             line["e2e"] = {"value": e["value"], "unit": UNIT, "h2d_bytes_per_step": e["h2d_bytes_per_step"], "d2h_bytes_per_step": e["d2h_bytes_per_step"],
                            "ms_per_step": e["ms_per_step"], "n_gpus_used": world, "sample": e["sample"], "note": e["note"]}
@@ -734,7 +768,7 @@ def run_ours(args):
                                    "ratio": "ours.value / the reference arm's value: computed by the driver from the two lines"}
             failed |= e.get("identical_to_oracle") is False
     elif rank == 0 and not args.no_decode:
-        e = decode_included(local, max(1, min(args.steps, 10)), 2, s_scale)
+        e = decode_included(local, args.steps, 2, s_scale)
         line["e2e"] = {"value": e["value"], "unit": UNIT, "h2d_bytes_per_step": e["h2d_bytes_per_step"], "d2h_bytes_per_step": e["d2h_bytes_per_step"],
                        "ms_per_step": e["ms_per_step"], "n_gpus_used": 1, "sample": e["sample"], "note": e["note"]}
         line["same_sample"] = {"ours": e, "reference": "bench.py --impl reference --steps %d --warmup %d on the same file (%s)" % (args.steps, args.warmup, e["sample"]),
@@ -748,18 +782,17 @@ def run_ours(args):
         line["parity_checked"] = parity_check(local, dev, min(args.scale, 1.0 / 16))
         failed |= not line["parity_checked"]["identical"]
     if rank == 0 and not args.no_legs:
-        st = max(1, min(args.steps, 3))
         legs = {}
         c2 = workload_cfg(args.scale)
-        legs["configs[2]"] = resident_leg(local, dev, c2, st, "BASELINE.json configs[2] on one GPU: configs[1] + exclude intervals (~5 %% of every chromosome) + -q 20 -s 15"
+        legs["configs[2]"] = resident_leg(local, dev, c2, args.steps, "BASELINE.json configs[2] on one GPU: configs[1] + exclude intervals (~5 %% of every chromosome) + -q 20 -s 15"
                                           + ("" if args.scale == 1.0 else " x scale %g" % args.scale), ctx_kw={"qual": 20, "sd_mult": 15}, exclude=exclude_intervals(c2))
         s4 = args.scale * 0.5                     # 100x at half the genome: 1.0e9 records, fits next to nothing else on one GPU
-        legs["configs[3]"] = resident_leg(local, dev, synth.config4(scale=s4), st, "BASELINE.json configs[3]: tumour-shaped 100x, planted translocations, x scale %g" % s4)
-        sr = resident_leg(local, dev, synth.config5(scale=args.stress_scale), st, "BASELINE.json configs[4] x scale %g: split-read refinement stress" % args.stress_scale)
+        legs["configs[3]"] = resident_leg(local, dev, synth.config4(scale=s4), args.steps, "BASELINE.json configs[3]: tumour-shaped 100x, planted translocations, x scale %g" % s4)
+        sr = resident_leg(local, dev, synth.config5(scale=args.stress_scale), args.steps, "BASELINE.json configs[4] x scale %g: split-read refinement stress" % args.stress_scale)
         sr_ms = sr["stage_ms"]["evidence"] + sr["stage_ms"]["refine"]
         sr["split_reads_refined_per_s"] = sr["n_sa"] / (sr_ms * 1e-3) if sr_ms > 0 else None
         legs["configs[4]"] = sr
-        legs["banded_alignment"] = align_leg(local)
+        legs["banded_alignment"] = align_leg(local, args.steps)
         line["legs"] = legs
         line["split_reads"] = {"value": sr["split_reads_refined_per_s"], "unit": "split reads refined/s", "note": "configs[4]: SA-tagged records / (evidence + refine stage time)"}
     if rank == 0:
@@ -844,7 +877,7 @@ def cpu_baseline_port(args):
     scale = min(sample_scale(args.steps, args.warmup), args.scale)
     cores = os.cpu_count()
     if os.path.exists(O.REF_BIN):
-        paths, n = sample_dataset(scale)
+        paths, n = sample_dataset(scale, index=True)
         O.ref_install_refgene(paths["refgene"])
         tmp = tempfile.mkdtemp(prefix="bkid_cpu_")
         t0 = time.perf_counter()
@@ -879,7 +912,7 @@ def run_reference(args):
     if not os.path.exists(O.REF_BIN):
         print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/BreakID_ref is not built (run __graft_entry__.build() where /root/reference exists)"}), flush=True)
         return
-    paths, n = sample_dataset(scale)
+    paths, n = sample_dataset(scale, index=True)
     O.ref_install_refgene(paths["refgene"])
     tmp = tempfile.mkdtemp(prefix="bkid_ref_")
     times = []
@@ -907,10 +940,17 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def _positive(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=_positive, default=5, help="timed steps of every measurement")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--scale", type=float, default=1.0, help="fraction of the hg19-shaped 30x workload per GPU")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -921,7 +961,10 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle comparison on configs[1] x 1/16")
     ap.add_argument("--stress-scale", type=float, default=1.0, help="fraction of the 1e7-SA-record stress workload")
     ap.add_argument("--py-dist", action="store_true", help="N > 1: use the Python-orchestrated exchanges instead of the library's NCCL path")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="single GPU: write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

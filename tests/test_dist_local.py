@@ -120,21 +120,27 @@ def test_multi_gpu_driver_matches_reference_binary(tmp_path, gpus, flags):
     built with the literal 3 of src/BreakID.cc:103 read from the environment, oracle/Makefile ref_s)."""
     import subprocess
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    sd_mult = 15 if "-s" in flags else None
+    ref = O.have_ref() and (sd_mult is None or os.path.exists(O.REF_BIN + "_s"))
     cfg = synth.SynthConfig(chrom_lens=[300000, 200000, 150000], n_tra=3, n_inv=2, n_dup=2, n_del=2, seed=23, sv_jitter=1)
     d = synth.generate(cfg)
     paths = bamio.write_dataset(str(tmp_path), d, genes_per_mb=25.0)
-    O.ref_index(paths["bam"])
-    O.ref_install_refgene(paths["refgene"])
-    sd_mult = 15 if "-s" in flags else None
-    r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None, sd_mult=sd_mult)
-    assert r.returncode == 0, r.stderr[-500:]
+    R.index(paths["bam"])
+    if ref:
+        O.ref_install_refgene(paths["refgene"])
+        r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None, sd_mult=sd_mult)
+        assert r.returncode == 0, r.stderr[-500:]
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", paths["bam"], "-o", str(tmp_path / "gpu"), "-n", paths["nib"], "-r", paths["refgene"], "-all", "-gpu", gpus] + flags,
                        timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, (g.stdout[-300:], g.stderr[-500:])
+    if not ref:
+        R.match_oracle(str(tmp_path / "gpu"), d, mode=int("-fast" in flags), qual=20 if "-q" in flags else None, sd_mult=sd_mult or 3)
+        assert len(R.fusion_all_rows(str(tmp_path / "gpu"))) >= 5
+        assert "communicator\tlocal" in open(str(tmp_path / "gpu") + "_b200_timings.txt").read()
+        return
     for suffix in ("_fusion.txt", "_fusion_all.txt"):
         a = open(str(tmp_path / "ref") + suffix).read()
         b = open(str(tmp_path / "gpu") + suffix).read()

@@ -294,21 +294,26 @@ def test_driver_call_files_match_reference_binary(tmp_path, mode):
     import os
     import subprocess
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    ref = O.have_ref()
     cfg = synth.SynthConfig(chrom_lens=[300000, 200000, 150000], n_tra=3, n_inv=2, n_dup=2, n_del=2, seed=21, sv_jitter=1)
     d = synth.generate(cfg)
     paths = bamio.write_dataset(str(tmp_path), d, genes_per_mb=25.0)
-    O.ref_index(paths["bam"])
-    O.ref_install_refgene(paths["refgene"])
+    R.index(paths["bam"])
     flags = ["-all"] + (["-fast"] if mode == "fast" else [])
-    r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast=(mode == "fast"))
-    assert r.returncode == 0, r.stderr[-500:]
+    if ref:
+        O.ref_install_refgene(paths["refgene"])
+        r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast=(mode == "fast"))
+        assert r.returncode == 0, r.stderr[-500:]
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", paths["bam"], "-o", str(tmp_path / "gpu"), "-n", paths["nib"], "-r", paths["refgene"]] + flags,
                        timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, g.stderr[-500:]
+    if not ref:
+        R.match_oracle(str(tmp_path / "gpu"), d, mode=int(mode == "fast"))
+        assert len(R.fusion_all_rows(str(tmp_path / "gpu"))) >= 5
+        return
     for suffix in ("_fusion.txt", "_fusion_all.txt"):
         a = open(str(tmp_path / "ref") + suffix).read()
         b = open(str(tmp_path / "gpu") + suffix).read()
@@ -317,6 +322,36 @@ def test_driver_call_files_match_reference_binary(tmp_path, mode):
     pa = open(str(tmp_path / "ref") + "_params.txt").read().replace(str(tmp_path / "ref"), "X")
     pb = open(str(tmp_path / "gpu") + "_params.txt").read().replace(str(tmp_path / "gpu"), "X")
     assert pa == pb
+
+
+@pytest.mark.parametrize("mode", ["ahc", "fast"])
+def test_driver_matches_stored_reference_call_files(tmp_path, mode):
+    """the BreakID driver on the dataset of tests/golden/make_golden.py against the files the reference binary wrote on it
+    (mini_ref_<mode>_fusion.txt, mini_ref_<mode>_fusion_all.txt, mini_ref_params.txt): byte for byte, gene annotation and
+    the gene-fusion filter included, with no reference needed"""
+    import os
+    import subprocess
+    import reference_calls as R
+    from breakid_b200 import bamio, synth
+    G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    cfg = synth.SynthConfig(chrom_lens=[120000, 90000], n_tra=2, n_inv=1, n_dup=1, n_del=1, seed=33, min_sv_sep=5000, sv_jitter=1,
+                            chimeric_frac=0.02)                                   # make_golden.mini_cfg()
+    d = synth.generate(cfg)
+    z = np.load(os.path.join(G, "mini.npz"))                                     # the records the reference ran on
+    assert all(np.array_equal(d.cols[k].numpy().view(z["col_" + k].dtype), z["col_" + k]) for k in ("flag", "mapq", "tid", "pos", "mtid", "mpos", "isize", "endpos"))
+    assert np.array_equal(synth.name_hash_ids(d.cols["name_id"]).numpy().view(np.uint64).reshape(-1), z["name_hash"])
+    paths = bamio.write_dataset(str(tmp_path), d, random_qual=False, genes_per_mb=40.0)
+    assert open(paths["refgene"]).read() == open(os.path.join(G, "mini_refGene.txt")).read()
+    R.index(paths["bam"])
+    drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
+    out = str(tmp_path / mode)
+    g = subprocess.run([drv, "-i", paths["bam"], "-o", out, "-n", paths["nib"], "-r", paths["refgene"], "-all"] + (["-fast"] if mode == "fast" else []),
+                       timeout=600, capture_output=True, text=True)
+    assert g.returncode == 0, g.stderr[-500:]
+    for suffix in ("_fusion.txt", "_fusion_all.txt"):
+        assert open(out + suffix).read() == open(os.path.join(G, "mini_ref_%s%s" % (mode, suffix))).read(), suffix
+    exp = open(os.path.join(G, "mini_ref_params.txt")).read()                     # stored from the AHC run (out_file TMP/ahc)
+    assert open(out + "_params.txt").read().replace(str(tmp_path), "TMP") == exp.replace("TMP/ahc", "TMP/" + mode)
 
 
 @pytest.mark.parametrize("mode", [0, 1])
@@ -520,25 +555,29 @@ def test_driver_config4_tumour_fusions(tmp_path, flags):
     import os
     import subprocess
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    ref = O.have_ref()
     cfg = synth.SynthConfig(chrom_lens=[260000, 220000, 180000, 140000], coverage=100.0, n_tra=10, n_inv=0, n_dup=0, n_del=0,
                             span_per_sv=40, split_per_sv=20, seed=44, sv_jitter=1)
     d = synth.generate(cfg)
     paths = bamio.write_dataset(str(tmp_path), d, genes_per_mb=30.0)
-    O.ref_index(paths["bam"])
-    O.ref_install_refgene(paths["refgene"])
-    r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], extra=flags)
-    assert r.returncode == 0, r.stderr[-500:]
+    R.index(paths["bam"])
+    if ref:
+        O.ref_install_refgene(paths["refgene"])
+        r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], extra=flags)
+        assert r.returncode == 0, r.stderr[-500:]
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", paths["bam"], "-o", str(tmp_path / "gpu"), "-n", paths["nib"], "-r", paths["refgene"], "-all"] + flags,
                        timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, g.stderr[-500:]
-    for suffix in ("_fusion.txt", "_fusion_all.txt"):
-        a = open(str(tmp_path / "ref") + suffix).read()
-        b = open(str(tmp_path / "gpu") + suffix).read()
-        assert a == b, (suffix, flags)
+    if ref:
+        for suffix in ("_fusion.txt", "_fusion_all.txt"):
+            a = open(str(tmp_path / "ref") + suffix).read()
+            b = open(str(tmp_path / "gpu") + suffix).read()
+            assert a == b, (suffix, flags)
+    else:
+        R.match_oracle(str(tmp_path / "gpu"), d, mode=int("-fast" in flags), qual=int(flags[flags.index("-q") + 1]) if "-q" in flags else None)
     rows = open(str(tmp_path / "gpu") + "_fusion_all.txt").read().splitlines()[1:]
     assert len(rows) >= 8 and all(x.split("\t")[0] == "Translocation" for x in rows)
     fused = [x for x in open(str(tmp_path / "gpu") + "_fusion.txt").read().splitlines()[1:]]
@@ -620,9 +659,9 @@ def test_driver_exclude_bed_matches_reference_on_prefiltered_bam(tmp_path):
     import subprocess
     import torch
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    ref = O.have_ref()
     cfg = synth.SynthConfig(chrom_lens=[300000, 200000, 150000], n_tra=3, n_inv=2, n_dup=2, n_del=2, seed=21, sv_jitter=1)
     d = synth.generate(cfg)
     iv = _exclude_intervals(d, np.random.RandomState(4))
@@ -645,16 +684,20 @@ def test_driver_exclude_bed_matches_reference_on_prefiltered_bam(tmp_path):
     d2 = synth.SynthData(cfg=cfg, cols={k: v[kt] for k, v in d.cols.items()}, sa_rec=new_index[d.sa_rec[sa_keep]],
                          cig_off=mkoff(lens(d.cig_off)), cig_ops=parts(d.cig_off, d.cig_ops), sa_off=mkoff(lens(d.sa_off)), sa_txt=parts(d.sa_off, d.sa_txt), truth=d.truth)
     filt = bamio.write_dataset(str(tmp_path / "filt"), d2, genes_per_mb=25.0)
-    O.ref_index(filt["bam"]); O.ref_index(full["bam"])
-    O.ref_install_refgene(full["refgene"])
-    r = O.ref_run_binary(filt["bam"], str(tmp_path / "ref"), filt["nib"])
-    assert r.returncode == 0, r.stderr[-500:]
+    R.index(filt["bam"]); R.index(full["bam"])
+    if ref:
+        O.ref_install_refgene(full["refgene"])
+        r = O.ref_run_binary(filt["bam"], str(tmp_path / "ref"), filt["nib"])
+        assert r.returncode == 0, r.stderr[-500:]
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", full["bam"], "-o", str(tmp_path / "gpu"), "-n", full["nib"], "-r", full["refgene"], "-all", "-x", str(tmp_path / "ex.bed")],
                        timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, g.stderr[-500:]
-    for suffix in ("_fusion.txt", "_fusion_all.txt"):
-        assert open(str(tmp_path / "ref") + suffix).read() == open(str(tmp_path / "gpu") + suffix).read(), suffix
+    if ref:
+        for suffix in ("_fusion.txt", "_fusion_all.txt"):
+            assert open(str(tmp_path / "ref") + suffix).read() == open(str(tmp_path / "gpu") + suffix).read(), suffix
+    else:
+        R.match_oracle(str(tmp_path / "gpu"), d2, check_w=False)
     assert len(open(str(tmp_path / "gpu") + "_fusion_all.txt").read().splitlines()) >= 4
 
 
@@ -834,20 +877,25 @@ def test_driver_sd_multiplier_matches_patched_reference(tmp_path, flags, sd_mult
     import os
     import subprocess
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
-    if not O.have_ref() or not os.path.exists(O.REF_BIN + "_s"):
-        pytest.skip("oracle/_ref/BreakID_ref_s not built (needs /root/reference at build time)")
+    ref = O.have_ref() and os.path.exists(O.REF_BIN + "_s")
     cfg = synth.SynthConfig(chrom_lens=[300000, 200000, 150000], n_tra=3, n_inv=2, n_dup=2, n_del=2, seed=29, sv_jitter=1)
     d = synth.generate(cfg)
     paths = bamio.write_dataset(str(tmp_path), d, genes_per_mb=25.0)
-    O.ref_index(paths["bam"])
-    O.ref_install_refgene(paths["refgene"])
-    r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None, sd_mult=sd_mult)
-    assert r.returncode == 0, r.stderr[-500:]
-    r3 = O.ref_run_binary(paths["bam"], str(tmp_path / "ref3"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None)
+    R.index(paths["bam"])
+    if ref:
+        O.ref_install_refgene(paths["refgene"])
+        r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None, sd_mult=sd_mult)
+        assert r.returncode == 0, r.stderr[-500:]
+        r3 = O.ref_run_binary(paths["bam"], str(tmp_path / "ref3"), paths["nib"], fast="-fast" in flags, qual=20 if "-q" in flags else None)
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", paths["bam"], "-o", str(tmp_path / "gpu"), "-n", paths["nib"], "-r", paths["refgene"], "-all"] + flags, timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, g.stderr[-500:]
+    if not ref:
+        mean, sd, dist = R.match_oracle(str(tmp_path / "gpu"), d, mode=int("-fast" in flags), qual=20 if "-q" in flags else None, sd_mult=sd_mult)
+        assert "%g" % dist != "%g" % O.dist(mean, sd)                  # the flag really changes w
+        return
     for suffix in ("_fusion.txt", "_fusion_all.txt"):
         assert open(str(tmp_path / "ref") + suffix).read() == open(str(tmp_path / "gpu") + suffix).read(), suffix
     pa = open(str(tmp_path / "ref") + "_params.txt").read().replace(str(tmp_path / "ref"), "X")

@@ -29,24 +29,29 @@ def test_multi_gpu_driver_over_nccl_matches_reference_binary(tmp_path, flags):
     the call files must be byte-identical to the reference CPU binary."""
     import torch
     import oracle_py as O
+    import reference_calls as R
     from breakid_b200 import bamio, synth
     n = min(torch.cuda.device_count(), 8)
     if n < 2:
         pytest.skip("needs >= 2 GPUs")
-    if not O.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+    ref = O.have_ref()
     cfg = synth.SynthConfig(chrom_lens=[300000, 200000, 150000], n_tra=3, n_inv=2, n_dup=2, n_del=2, seed=29, sv_jitter=1)
     d = synth.generate(cfg)
     paths = bamio.write_dataset(str(tmp_path), d, genes_per_mb=25.0)
-    O.ref_index(paths["bam"])
-    O.ref_install_refgene(paths["refgene"])
-    r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags)
-    assert r.returncode == 0, r.stderr[-2000:]
+    R.index(paths["bam"])
+    if ref:
+        O.ref_install_refgene(paths["refgene"])
+        r = O.ref_run_binary(paths["bam"], str(tmp_path / "ref"), paths["nib"], fast="-fast" in flags)
+        assert r.returncode == 0, r.stderr[-2000:]
     drv = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "breakid_b200", "host", "BreakID")
     g = subprocess.run([drv, "-i", paths["bam"], "-o", str(tmp_path / "gpu"), "-n", paths["nib"], "-r", paths["refgene"], "-all", "-gpu", "0-%d" % (n - 1)] + flags,
                        timeout=600, capture_output=True, text=True)
     assert g.returncode == 0, (g.stdout[-2000:], g.stderr[-2000:])
     assert "communicator\tnccl" in open(str(tmp_path / "gpu") + "_b200_timings.txt").read()
+    if not ref:
+        R.match_oracle(str(tmp_path / "gpu"), d, mode=int("-fast" in flags))
+        assert len(R.fusion_all_rows(str(tmp_path / "gpu"))) >= 5
+        return
     for suffix in ("_fusion.txt", "_fusion_all.txt"):
         a = open(str(tmp_path / "ref") + suffix).read()
         assert a == open(str(tmp_path / "gpu") + suffix).read(), suffix
