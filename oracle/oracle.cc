@@ -537,11 +537,20 @@ struct Comp {
   int merges;
   int hi_oc_leaf;                 /* highest global leaf index NOT in this component (-1 if none) */
   int head_j; double head_d;      /* current best event */
+  long flag_decisions;            /* decisions the device's speculative pass flags (orc_model_ahc_flags) */
 };
 }  // namespace
 
 static long g_model_exc_taken = 0, g_model_exc_blocked = 0;
 void orc_model_ahc_counters(long *taken, long *blocked) { *taken = g_model_exc_taken; *blocked = g_model_exc_blocked; }
+
+/* Flag predictor.  The device's speculative pass (bkid_cluster.cuh ahc_find_best<false>) flags a component when a tail
+ * exception needs the out-of-component sentinel and that cannot be settled statically: j is a merged node, unless t2 is a
+ * leaf and some out-of-component leaf index lies above it.  Up to its first such decision a component takes the same path
+ * here and on the device, so "flagged" == "at least one such decision in the model".  Counts of the last
+ * orc_model_ahc_tree call: components flagged, and all such decisions. */
+static long g_model_flag_comps = 0, g_model_flag_decisions = 0;
+void orc_model_ahc_flags(long *flagged_comps, long *decisions) { *flagged_comps = g_model_flag_comps; *decisions = g_model_flag_decisions; }
 
 long orc_model_ahc_tree(long n, const double *x, const double *y, long thr,
                         int32_t *is_root, int32_t *merged_a, int32_t *merged_b)
@@ -563,7 +572,7 @@ long orc_model_ahc_tree(long n, const double *x, const double *y, long thr,
       while (s2 < oy.size()) {
         size_t e2 = s2 + 1;
         while (e2 < oy.size() && !(y[oy[e2]] - y[oy[e2 - 1]] > (double)thr)) ++e2;
-        Comp c; c.merges = 0; c.head_j = -1; c.head_d = DBL_MAX; c.hi_oc_leaf = -1;
+        Comp c; c.merges = 0; c.head_j = -1; c.head_d = DBL_MAX; c.hi_oc_leaf = -1; c.flag_decisions = 0;
         c.leaves.assign(oy.begin() + s2, oy.begin() + e2);
         std::sort(c.leaves.begin(), c.leaves.end());
         for (int l : c.leaves) comp_of[l] = (int)comps.size();
@@ -613,6 +622,7 @@ long orc_model_ahc_tree(long n, const double *x, const double *y, long thr,
     /* in-component part of the tail test */
     for (int t : ts) if (t > t2 && t != t1 && !(rowd(c, j, t) < dmin)) return;
     /* out-of-component sentinel */
+    if (j >= cl && !(t2 < cl && c.hi_oc_leaf > c.leaves[t2])) ++c.flag_decisions;
     bool sentinel;
     if (j < cl) sentinel = lo_oc[c.leaves[j]] > c.leaves[t2];
     else if (t2 >= cl) sentinel = (nj.grank - c.nodes[t2].grank) > (long)(nj.lrank - c.nodes[t2].lrank);
@@ -667,6 +677,8 @@ long orc_model_ahc_tree(long n, const double *x, const double *y, long thr,
       if (c.nodes[j].is_root && (c.nodes[j].best_t == first || c.nodes[j].best_t == second)) find_best(c, j);
     comp_head(c);
   }
+  g_model_flag_comps = g_model_flag_decisions = 0;
+  for (const Comp &c : comps) { g_model_flag_comps += c.flag_decisions > 0; g_model_flag_decisions += c.flag_decisions; }
   long nn = (long)g.size();
   for (long i = 0; i < nn; ++i) { is_root[i] = g[i].root; merged_a[i] = g[i].a; merged_b[i] = g[i].b; }
   return nn;
@@ -682,6 +694,17 @@ long orc_model_cluster_ahc(long n, const uint32_t *p1, const uint32_t *p2, doubl
   return tree_to_clusters(n, nn, r.data(), a.data(), b.data(), out_idx, out_cluster, roots);
 }
 
+
+/* Per-bucket AHC of orc_run and orc_shard_bucket_clusters: the literal restatement by default; orc_set_ahc_model(1) switches
+ * to the component model, which is pinned to the literal form by the CPU suite and is the only one fast enough for buckets
+ * of thousands of points (the literal form is O(N^3)). */
+static int g_ahc_model = 0;
+void orc_set_ahc_model(int on) { g_ahc_model = on != 0; }
+static long bucket_ahc(long n, const uint32_t *p1, const uint32_t *p2, double thr, uint32_t *out_idx, int32_t *out_cluster, int *roots)
+{
+  return g_ahc_model ? orc_model_cluster_ahc(n, p1, p2, thr, out_idx, out_cluster, roots)
+                     : orc_cluster_ahc(n, p1, p2, thr, out_idx, out_cluster, roots);
+}
 
 /* ==========================================================================================
  * Refinement: a7 cluster summary, a8 split-read evidence, a9 vote, a10 depth/AF/type, a11 nib.
@@ -1039,7 +1062,7 @@ long orc_run(long n, const uint16_t *flag, const uint8_t *mapq, const int32_t *t
       for (long i = 0; i < nm; ++i) { q1[i] = p1[idx[i]]; q2[i] = p2[idx[i]]; }
       int roots = 0;
       long nc = mode ? orc_cluster_fast(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots)
-                     : orc_cluster_ahc(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots);
+                     : bucket_ahc(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots);
       /* a7: per-cluster summary (src/BreakID.cc:222-352); order inside a cluster does not matter */
       std::map<long, std::vector<long>> members;
       for (long i = 0; i < nc; ++i) members[cl[i]].push_back(s + idx[cidx[i]]);
@@ -1223,7 +1246,7 @@ long orc_shard_bucket_clusters(long np, const orc_pair *pairs, double dist, int 
       for (long i = 0; i < nm; ++i) { q1[i] = p1[idx[i]]; q2[i] = p2[idx[i]]; }
       int roots = 0;
       long nc = mode ? orc_cluster_fast(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots)
-                     : orc_cluster_ahc(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots);
+                     : bucket_ahc(nm, q1.data(), q2.data(), dist, cidx.data(), cl.data(), &roots);
       std::map<long, std::vector<long>> members;
       for (long i = 0; i < nc; ++i) members[cl[i]].push_back(s + idx[cidx[i]]);
       for (auto &kv : members) {

@@ -49,8 +49,9 @@ def _bytes_tensor(ptr, n, row, free):
 class OracleEngine:
     device = torch.device("cpu")
 
-    def __init__(self, hb, nibs=None, qual=20):
-        self.hb, self.nibs, self.qual = hb, nibs, qual
+    def __init__(self, hb, nibs=None, qual=20, ahc_model=False):
+        """ahc_model: cluster() runs the component model of AHC instead of the literal O(N^3) form (see O.ahc_model)"""
+        self.hb, self.nibs, self.qual, self.ahc_model = hb, nibs, qual, ahc_model
         self.o = _lib()
         self.rank_table = np.zeros((len(hb.target_names) + 1) ** 2, np.int32)
         self.o.orc_bucket_rank_table(len(hb.target_names), O._names(hb), self.rank_table)
@@ -105,7 +106,11 @@ class OracleEngine:
 
     def cluster(self, d, mode):
         out = vp()
-        n = self.o.orc_shard_bucket_clusters(self.pairs.shape[0], self.pairs.ctypes.data, d, mode, C.byref(out))
+        self.o.orc_set_ahc_model(1 if self.ahc_model else 0)
+        try:
+            n = self.o.orc_shard_bucket_clusters(self.pairs.shape[0], self.pairs.ctypes.data, d, mode, C.byref(out))
+        finally:
+            self.o.orc_set_ahc_model(0)
         self._cl = _bytes_tensor(out, n, 192, self.o.orc_free)
 
     def clusters(self):

@@ -64,6 +64,9 @@ def olib():
         for f in (o.orc_ahc_tree, o.orc_model_ahc_tree):
             f.restype = L
             f.argtypes = [L, f64p, f64p, L, i32p, i32p, i32p]
+        o.orc_set_ahc_model.argtypes = [I]
+        o.orc_model_ahc_flags.argtypes = [C.POINTER(L), C.POINTER(L)]
+        o.orc_model_heapsort_count.restype = L
         o.orc_is_complementary.argtypes = [C.c_char_p, C.c_char_p, I]
         rec = [L, u16p, u8p, i32p, i32p, i32p, u64p, L, u32p, u32p, u32p, u32p, u8p, u32p, u8p]
         o.orc_find_sa_reads.restype = L
@@ -187,6 +190,31 @@ def cluster(mode, p1, p2, thr, model=False):
     f = olib().orc_cluster_fast if mode else (olib().orc_model_cluster_ahc if model else olib().orc_cluster_ahc)
     n = f(p1.shape[0], p1, p2, thr, oi, oc, C.byref(r))
     return oi[:n], oc[:n], r.value
+
+
+class ahc_model:
+    """inside the block, the per-bucket AHC of run() and of OracleEngine.cluster is the component model instead of the
+    literal O(N^3) restatement"""
+
+    def __enter__(self):
+        olib().orc_set_ahc_model(1)
+
+    def __exit__(self, *a):
+        olib().orc_set_ahc_model(0)
+
+
+def ahc_flags(p1, p2, thr):
+    """(components the device's speculative AHC pass flags, decisions that flag them) on these points (post-mask order),
+    predicted by the component model"""
+    cluster(0, p1, p2, thr, model=True)
+    f, d = L(), L()
+    olib().orc_model_ahc_flags(C.byref(f), C.byref(d))
+    return f.value, d.value
+
+
+def heapsort_count():
+    """depth-exhausted segments the sort model has finished with the literal heapsort so far (cumulative)"""
+    return olib().orc_model_heapsort_count()
 
 
 def banded_edit(q: bytes, r: bytes, w: int) -> int:

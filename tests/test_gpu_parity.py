@@ -388,19 +388,28 @@ def test_sa_rows_match_oracle(small_data):
     c.close()
 
 
-def test_ahc_large_bucket_rank_form(ctx1):
+def test_ahc_large_bucket_rank_form(ctx1, monkeypatch, capfd):
     """one bucket with > 4096 points (global-memory rank-form replay) incl. exact cross-component ties; the
-    oracle side is the component model (proven equal to the literal O(N^3) restatement in the CPU suite)"""
+    oracle side is the component model (proven equal to the literal O(N^3) restatement in the CPU suite).  The rank form
+    only serves buckets without flagged components: the count the library prints with BKID_DEBUG_TIMING=1 says so.  (With
+    7-spaced offsets from a range of 6, the 9 000-point bucket had 11 flagged components and took ahc_bucket_exact;
+    tests/test_cluster_forms.py covers that form.)"""
     import oracle_py as O
+    from test_cluster_forms import flagged_witness
+    monkeypatch.setenv("BKID_DEBUG_TIMING", "1")
     rng = np.random.RandomState(123)
-    for n, spread in ((5000, 40), (9000, 6)):
+    for n, spread in ((5000, 40), (9000, 16)):
         k = n // 12
         cx = np.sort(rng.choice(np.arange(0, 40_000_000, 5000), k, replace=False)); cy = rng.randint(0, 40_000_000, k)
         a = rng.randint(0, k, n)
         x = (cx[a] + rng.randint(0, spread, n) * 7).astype(np.uint32); y = (cy[a] + rng.randint(0, spread, n) * 7).astype(np.uint32)
         o = np.argsort(x, kind="stable"); x = np.ascontiguousarray(x[o]); y = np.ascontiguousarray(y[o])
         ei, ec, er = O.cluster(0, x, y, 1243.15, model=True)
+        assert O.ahc_flags(x, y, 1243.15)[0] == 0
+        capfd.readouterr()
         gi, gc, gr = ctx1.op_cluster(0, x, y, 1243.15)
+        seen = flagged_witness(capfd.readouterr().err)
+        assert len(seen) == 1 and seen[0][1] == 0 and seen[0][2] == n, seen
         assert np.array_equal(ei, gi) and np.array_equal(ec, gc) and er == gr, n
 
 
