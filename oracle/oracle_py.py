@@ -267,9 +267,9 @@ def run(hb, nibs=None, qual=20, times=2, mode=0, sd_mult=3):
 def _run(hb, nibs, qual, times, mode):
     c, s = hb.cols, hb.side
     nt = len(hb.target_names)
-    if nibs is not None:
-        keep = [np.ascontiguousarray(p, np.uint8) for p, _ in nibs]
-        ptrs = (C.c_void_p * nt)(*[k.ctypes.data for k in keep])
+    if nibs is not None:                          # an entry (None, 0): no nib for that tid, its 41-mers stay empty
+        keep = [None if p is None else np.ascontiguousarray(p, np.uint8) for p, _ in nibs]
+        ptrs = (C.c_void_p * nt)(*[None if k is None else k.ctypes.data for k in keep])
         lens = (C.c_uint64 * nt)(*[int(l) for _, l in nibs])
     else:
         ptrs, lens = None, None
