@@ -280,7 +280,7 @@ EXPORTS = ["bkid_abi_version", "bkid_last_error", "bkid_default_params", "bkid_c
            "bkid_shard_finish", "bkid_fetch_bucket_ranks", "bkid_device_copy",
            "bkid_push_bgzf", "bkid_push_bgzf_range", "bkid_get_decode_stats", "bkid_fetch_column", "bkid_set_exclude", "bkid_device_gather_rows", "bkid_op_banded_align", "bkid_profile_kernels", "bkid_profile_report",
            "bkid_comm_nccl_unique_id", "bkid_comm_nccl_init", "bkid_comm_nccl_init_all", "bkid_comm_local_create", "bkid_comm_destroy", "bkid_dist_run", "bkid_dist_run_threads",
-           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table"]
+           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table", "bkid_sort_records"]
 
 CAND_BYTES = 48
 SAROW_BYTES = 88
@@ -313,6 +313,7 @@ def cuda_lib():
         L.bkid_get_decode_stats.argtypes = [vp, C.POINTER(DecodeStats)]
         L.bkid_fetch_column.argtypes = [vp, C.c_char_p, vp, C.c_int64, C.POINTER(C.c_int64)]
         L.bkid_reset.argtypes = [vp]
+        L.bkid_sort_records.argtypes = [vp, C.POINTER(C.c_int32)]
         L.bkid_insert_stats.argtypes = [vp, dp, dp]
         L.bkid_scan.argtypes = [vp, C.c_double, i64p]
         L.bkid_cluster.argtypes = [vp, C.c_double, C.c_int, i64p]
@@ -552,6 +553,13 @@ class Context:
 
     def reset(self):
         self._chk(self.lib.bkid_reset(self.ctx))
+
+    def sort_records(self) -> bool:
+        """coordinate-sort the records pushed so far on the device (``bkid_sort_records``); True when they already were
+        in order (nothing moved)"""
+        w = C.c_int32()
+        self._chk(self.lib.bkid_sort_records(self.ctx, C.byref(w)))
+        return bool(w.value)
 
     def insert_stats(self):
         m, s = C.c_double(), C.c_double()

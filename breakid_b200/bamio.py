@@ -1,7 +1,8 @@
 """Minimal BAM *writer* for synthetic workloads (test / bench tooling, not on the hot path).
 
-Writes the coordinate-sorted record batch of ``synth.SynthData`` as a real BGZF-compressed BAM so
-that the unmodified reference CPU binary can be run on byte-identical input.  The `.bai` index is
+Writes the record batch of ``synth.SynthData`` in its own record order as a real BGZF-compressed BAM so
+that the unmodified reference CPU binary can be run on byte-identical input.  ``sort_order`` is the @HD SO: tag
+("coordinate" for the batches synth.generate makes; "unsorted" / "queryname" for synth.permute'd ones).  The `.bai` index is
 NOT written here: tests build it with ``oracle/_ref/bamindex`` (the reference's own vendored
 htslib), the product only checks that the index file exists (reference src/BreakID.cc:411-416).
 """
@@ -39,8 +40,9 @@ def reg2bin(beg: np.ndarray, end: np.ndarray) -> np.ndarray:
 
 
 def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: int = 1,
-              chunk: int = 200_000, sa_seq=None) -> None:
-    """``sa_seq`` = optional seq table (seq_off / seq4 / seq_len, see synth.split_read_sequences): real read bases for
+              chunk: int = 200_000, sa_seq=None, sort_order: str = "coordinate") -> None:
+    """``sort_order`` = the @HD SO: value; the records are written in the batch's order whatever it says.
+    ``sa_seq`` = optional seq table (seq_off / seq4 / seq_len, see synth.split_read_sequences): real read bases for
     the SA-tagged records (all other records carry a constant sequence)."""
     cfg = d.cfg
     L = cfg.read_len
@@ -59,7 +61,7 @@ def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: in
     rng = np.random.RandomState(cfg.seed + 12345)
 
     # header
-    text = "@HD\tVN:1.4\tSO:coordinate\n" + "".join(
+    text = "@HD\tVN:1.4\tSO:%s\n" % sort_order + "".join(
         "@SQ\tSN:%s\tLN:%d\n" % (synth.chrom_name(t), l) for t, l in enumerate(cfg.chrom_lens))
     hdr = b"BAM\x01" + struct.pack("<i", len(text)) + text.encode() + struct.pack("<i", len(cfg.chrom_lens))
     for t, l in enumerate(cfg.chrom_lens):
@@ -152,7 +154,7 @@ def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: in
 
 
 def write_dataset(dirpath: str, d: synth.SynthData, random_qual: bool = True, nib: bool = True,
-                  genes_per_mb: float = 4.0) -> dict:
+                  genes_per_mb: float = 4.0, sort_order: str = "coordinate") -> dict:
     """Lay down everything a BreakID run needs: <dir>/reads.bam, <dir>/nib/{ref_names.txt,
     hg19_<chr>.nib}, <dir>/ref_files/refGene.txt.  Returns the paths."""
     import os
@@ -160,7 +162,7 @@ def write_dataset(dirpath: str, d: synth.SynthData, random_qual: bool = True, ni
     os.makedirs(os.path.join(dirpath, "ref_files"), exist_ok=True)
     cfg = d.cfg
     bam = os.path.join(dirpath, "reads.bam")
-    write_bam(bam, d, random_qual=random_qual)
+    write_bam(bam, d, random_qual=random_qual, sort_order=sort_order)
     synth.write_ref_names(os.path.join(dirpath, "nib", "ref_names.txt"), len(cfg.chrom_lens))
     if nib:
         for t, l in enumerate(cfg.chrom_lens):

@@ -1493,6 +1493,7 @@ __global__ void pair_xy(const bkid_pair *__restrict__ pairs, long long np, uint3
 #include "bkid_refine.cuh"
 #include "bkid_align.cuh"
 #include "bkid_api.cuh"
+#include "bkid_sort.cuh"
 #include "bkid_dist.cuh"
 #include "bkid_bamdec.cuh"
 #include "bkid_align_api.cuh"

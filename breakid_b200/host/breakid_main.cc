@@ -11,7 +11,9 @@
 //   * -gpu 0,1,2,...  several GPUs of one box: one host thread and one context per device, every rank inflates and
 //     decodes its own BGZF block range of the BAM (genomic-bin sharding of the file itself), the exchanges between the
 //     ranks are NCCL calls inside the library (bkid_dist_run).  A device may be named more than once (-gpu 0,0,0): the
-//     ranks then share it and exchange through device copies -- that is how the path is tested on a one-GPU box.
+//     ranks then share it and exchange through device copies -- that is how the path is tested on a one-GPU box;
+//   * -sort  the BAM may be in any record order (e.g. read-name grouped, as bwa mem | samblaster writes it): the records are
+//     coordinate sorted on the device after decode (bkid_sort_records), and no .bai is required.  One GPU only.
 // Host work: BAM decode (bam_reader.cc), .nib loading, refGene annotation, the final unstable sort
 // by N_DRP and file writing.  Everything between decode and the cluster records runs on the GPU.
 #include <getopt.h>
@@ -51,6 +53,7 @@ static const char *kHelp =
     "     \t -x         \t exclude regions (BED: chrom, start, end): records starting there are ignored [none]\n "
     "     \t -validate  \t split reads count only if their clipped bases align where the SA tag says (needs nib files) [off]\n "
     "     \t -threads   \t BAM decode threads [8]\n "
+    "     \t -sort      \t input BAM in any record order: sort on the GPU, no index needed (one GPU only) [off]\n "
     "     \t -gpu       \t CUDA device, or a list / range such as 0,1 or 0-7 (one rank per entry, NCCL between them) [0]\n ";
 
 static const char *kFusion[] = {"Unknown", "Translocation", "Inversion", "Duplication", "Deletion"};
@@ -90,7 +93,7 @@ static void write_row(std::ofstream &o, const CallRow &r, const std::vector<std:
 // shared by the single-GPU and the multi-GPU path.  `extra` writes the <o>_b200_timings.txt body.
 template <typename Extra>
 static void finish_and_write(const std::string &inp, const std::string &out, const std::string &refgene, const std::vector<std::string> &names,
-                             const std::vector<bkid_cluster_rec> &cl, bool filter, int qual, double dist, bool reached_breakpoint_stage, double t_start,
+                             const std::vector<bkid_cluster_rec> &cl, bool filter, bool need_index, int qual, double dist, bool reached_breakpoint_stage, double t_start,
                              int64_t n_pairs, int64_t n_masked, int64_t n_clustered, int64_t n_clusters, double t_scan, double t_cluster, double t_bp, Extra extra)
 {
   std::vector<Transcript> tx;
@@ -98,7 +101,7 @@ static void finish_and_write(const std::string &inp, const std::string &out, con
   std::vector<CallRow> rows;
   if (reached_breakpoint_stage) {
     // the reference opens the index and refGene as soon as one bucket reaches the break-point stage
-    if (!exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
+    if (need_index && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
       std::cerr << "Error: please index bam-file first:\t" << inp << std::endl;                     // src/BreakID.cc:412-416
       exit(1);
     }
@@ -156,11 +159,11 @@ int main(int argc, char *argv[])
   double t_start = now_s();
   static struct option longopts[] = {
       {"help", 0, 0, 'h'}, {"i", 1, 0, 1}, {"o", 1, 0, 2}, {"q", 1, 0, 3}, {"n", 1, 0, 4}, {"fast", 0, 0, 5}, {"t", 1, 0, 6},
-      {"all", 0, 0, 7}, {"s", 1, 0, 8}, {"r", 1, 0, 9}, {"threads", 1, 0, 10}, {"gpu", 1, 0, 11}, {"x", 1, 0, 12}, {"validate", 0, 0, 13}, {0, 0, 0, 0}};
+      {"all", 0, 0, 7}, {"s", 1, 0, 8}, {"r", 1, 0, 9}, {"threads", 1, 0, 10}, {"gpu", 1, 0, 11}, {"x", 1, 0, 12}, {"validate", 0, 0, 13}, {"sort", 0, 0, 14}, {0, 0, 0, 0}};
   std::string inp, out, nib_dir, refgene, exclude_bed;
   int qual = 20, times = 2, sd_mult = 3, threads = 8, gpu = 0;
   std::vector<int> gpus;
-  bool fast = false, filter = true, validate = false;
+  bool fast = false, filter = true, validate = false, sort = false;
   int opt, li;
   optind = 0;
   opterr = 0;
@@ -192,6 +195,7 @@ int main(int argc, char *argv[])
       }
       case 12: exclude_bed = optarg; break;
       case 13: validate = true; break;
+      case 14: sort = true; break;
       case '?':
         if (optopt == 0 && optind > 0 && (!strcmp(argv[optind - 1], "-?") || !strcmp(argv[optind - 1], "-help"))) { std::cerr << kHelp; exit(1); }
         std::cerr << kHelp;
@@ -201,6 +205,10 @@ int main(int argc, char *argv[])
   }
   if (inp.empty() || out.empty()) { std::cerr << kHelp; std::cerr << "Error: input- and output file is required.\n"; exit(1); }
   if (nib_dir.empty()) { std::cerr << kHelp; std::cerr << "Error: nib file's root dir is required.\n"; exit(1); }
+  if (sort && gpus.size() > 1) {
+    std::cerr << "Error: -sort works on one GPU only; sort the BAM first to use several (-gpu " << gpus.size() << " devices)\n";
+    exit(1);
+  }
   if (refgene.empty()) {
     const char *inst = getenv("BREAKID_INSTALLDIR");
     refgene = std::string(inst ? inst : ".") + "/ref_files/refGene.txt";
@@ -308,7 +316,7 @@ int main(int argc, char *argv[])
     cl.resize((size_t)n);
     int64_t pairs = 0, masked = 0, clustered = 0, nclusters = 0, records = 0;
     for (int r = 0; r < W; ++r) { bkid_timings t; bkid_get_timings(ctxs[r], &t); pairs += t.n_pairs; masked += t.n_masked; clustered += t.n_clustered; nclusters += t.n_clusters; records += nrec[r]; }
-    finish_and_write(inp, out, refgene, names, cl, filter, qual, dist[0], clustered > 0, t_start, pairs, masked, clustered, nclusters, t_run, 0.0, 0.0,
+    finish_and_write(inp, out, refgene, names, cl, filter, true, qual, dist[0], clustered > 0, t_start, pairs, masked, clustered, nclusters, t_run, 0.0, 0.0,
                      [&](std::ofstream &j) { j << "decoder\tdevice\nranks\t" << W << "\ncommunicator\t" << (distinct ? "nccl" : "local") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push
                                                 << "\nrun_s\t" << t_run << "\nrecords\t" << records << "\n"; });
     for (int r = 0; r < W; ++r) { bkid_comm_destroy(comms[r]); bkid_destroy(ctxs[r]); }
@@ -333,6 +341,13 @@ int main(int argc, char *argv[])
     bkid_get_decode_stats(ctx, &dst);
   }
   double t_push = now_s() - t_push0;
+  double t_sort = 0;
+  int32_t was_sorted = 1;
+  if (sort) {
+    double t1 = now_s();
+    if (bkid_sort_records(ctx, &was_sorted)) die("sort_records");
+    t_sort = now_s() - t1;
+  }
   double mean = 0, sd = 0;
   if (bkid_insert_stats(ctx, &mean, &sd)) die("insert_stats");
   std::cout << "the insert size mean: " << mean << ", the insert size sd:" << sd << " .\n";
@@ -352,7 +367,7 @@ int main(int argc, char *argv[])
   std::vector<bkid_cluster_rec> cl;
   double t_bp = 0;
   if (tm.n_clustered > 0) {
-    if (!exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
+    if (!sort && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
       std::cerr << "Error: please index bam-file first:\t" << inp << std::endl;                     // src/BreakID.cc:412-416
       exit(1);
     }
@@ -370,12 +385,13 @@ int main(int argc, char *argv[])
     cl.resize((size_t)n);
   }
   bkid_get_timings(ctx, &tm);
-  finish_and_write(inp, out, refgene, names, cl, filter, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
+  finish_and_write(inp, out, refgene, names, cl, filter, !sort, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
                    [&](std::ofstream &j) {
                      j << "decoder\t" << (host_decode ? "host" : "device") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ninflate_ms\t" << dst.inflate_ms << "\nboundaries_ms\t" << dst.boundaries_ms
                        << "\nextract_ms\t" << dst.extract_ms << "\ncompressed_bytes\t" << dst.compressed_bytes << "\nuncompressed_bytes\t" << dst.uncompressed_bytes << "\nrecords\t" << tm.n_records << "\nh2d_ms\t" << tm.h2d << "\nclassify_ms\t" << tm.classify << "\ninsert_stats_ms\t" << tm.insert_stats
                        << "\njoin_ms\t" << tm.join << "\nbucket_sort_ms\t" << tm.bucket_sort << "\nmask_ms\t" << tm.mask << "\ncluster_ms\t" << tm.cluster << "\nsummarize_ms\t" << tm.summarize
                        << "\nevidence_ms\t" << tm.evidence << "\nrefine_ms\t" << tm.refine << "\n";
+                     if (sort) j << "sort_ms\t" << t_sort * 1e3 << "\ninput_was_sorted\t" << was_sorted << "\n";
                    });
   bkid_destroy(ctx);
   if (bam) bkid_host_bam_free(bam);

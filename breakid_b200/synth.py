@@ -89,6 +89,35 @@ class SynthData:
         return int(self.cols["flag"].numel())
 
 
+def _segments(off: torch.Tensor, data: torch.Tensor, order: torch.Tensor):
+    """variable-length segments data[off[k]:off[k+1]] re-laid out in the row order `order` -> (new offsets, new data)"""
+    ln = (off[1:] - off[:-1])[order]
+    new_off = torch.zeros(order.numel() + 1, dtype=off.dtype, device=off.device)
+    new_off[1:] = torch.cumsum(ln, 0)
+    total = int(new_off[-1])
+    if total == 0:
+        return new_off, data[:0].clone()
+    seg = torch.repeat_interleave(torch.arange(order.numel(), device=off.device), ln)
+    src = off[:-1][order][seg] + (torch.arange(total, device=off.device) - new_off[:-1][seg])
+    return new_off, data[src]
+
+
+def permute(d: SynthData, order) -> SynthData:
+    """the same records in a new file order: new record i is old record order[i] (a permutation of range(n)).  The SA side
+    table is re-laid out in ascending new record index, as a decoder of the permuted file would list it."""
+    order = torch.as_tensor(order, dtype=torch.int64, device=d.cols["flag"].device)
+    assert order.numel() == d.n
+    new_of = torch.empty_like(order)
+    new_of[order] = torch.arange(d.n, dtype=torch.int64, device=order.device)
+    cols = {k: v[order] for k, v in d.cols.items()}
+    sa_new = new_of[d.sa_rec]
+    rows = torch.argsort(sa_new, stable=True)
+    cig_off, cig_ops = _segments(d.cig_off, d.cig_ops, rows)
+    sa_off, sa_txt = _segments(d.sa_off, d.sa_txt, rows)
+    return SynthData(cfg=d.cfg, cols=cols, sa_rec=sa_new[rows], cig_off=cig_off, cig_ops=cig_ops, sa_off=sa_off, sa_txt=sa_txt,
+                     truth=d.truth)
+
+
 def _digits(v: torch.Tensor):
     """decimal digit count of non-negative int64 tensor (>=1)."""
     n = torch.ones_like(v)

@@ -224,6 +224,26 @@ int bkid_push_bgzf_range(bkid_ctx *ctx, const uint8_t *file, uint64_t file_size,
                          uint64_t first_record_uoffset, int64_t first_block, int64_t end_block, int64_t *n_records,
                          uint64_t *first_record_uoff, uint64_t *next_record_uoff);
 int bkid_get_decode_stats(bkid_ctx *ctx, bkid_decode_stats *stats);
+/* Extension (the reference requires a coordinate-sorted, indexed BAM): put the records the context holds (every batch
+ * pushed so far) into coordinate order on the device.
+ * *was_sorted = 1: they already were non-decreasing in (tid as uint32, so tid -1 is last; pos).  Nothing moves: a file
+ *   sorted by any tool, with any tie order, runs exactly as it does without the call.
+ * Otherwise: stable sort (ties keep push order) by the lexicographic key (tid as uint32, pos + 1, flag & BAM_FREVERSE).
+ *   That is the order samtools 1.3.1 `sort` writes (the version the reference vendors): its key is
+ *   (uint64_t)tid << 32 | (pos + 1) << 1 | bam_is_rev under a stable merge sort, and the two keys agree for
+ *   pos + 1 < 2^30, which covers every human contig.
+ * Every dense column is permuted in the form the context holds it (narrow isize16 / span16 stay narrow), x_rec / sa_rec
+ * are renumbered, the sparse table and the SA side table (with cig_ops, sa_txt, oc_txt, seq4) are re-emitted in
+ * ascending new record index.  Like a push, the call invalidates every stage result; a push after it appends in push
+ * order (sort again).  A context holding borrowed device columns (bkid_push_batch_device) gets owned copies; the
+ * caller's memory is never written.
+ * Errors: a tid outside [-1, n_targets) or pos < -1 -> BKID_ERR_ARG; with 2^30 records or more, one target holding
+ * 2^30 records or more -> BKID_ERR_ARG.  All scratch is allocated before the first column is overwritten, so
+ * BKID_ERR_ARG and BKID_ERR_NOMEM leave the context exactly as it was.
+ * Device scratch (kept by the context for the next call), bytes per record: 24 (keys + push index, sort buffers)
+ * + 8 (packed row; 16 when a column is held wide) + 18 (slot maps, flags, offsets; only with sparse / SA rows or
+ * 2^30 records or more), plus about 2x the sparse and SA tables; a borrowed context adds its owned columns. */
+int bkid_sort_records(bkid_ctx *ctx, int32_t *was_sorted);
 /* parity-test getter: one input column of the context by name ("flag", "pos", "x_name_hash", "sa_txt", ...) */
 int bkid_fetch_column(bkid_ctx *ctx, const char *name, void *out, int64_t cap_bytes, int64_t *n_bytes);
 /* forget all records (keeps allocations) */
