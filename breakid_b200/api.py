@@ -265,6 +265,15 @@ def host_lib():
             fn.restype = rt
             fn.argtypes = [C.c_void_p]
         L.bkid_host_bgzf_close.argtypes = [C.c_void_p]
+        L.bkid_host_sam_open.restype = C.c_void_p
+        L.bkid_host_sam_open.argtypes = [C.c_char_p, C.c_char_p, C.c_int]
+        L.bkid_host_sam_parse.restype = C.c_void_p
+        L.bkid_host_sam_parse.argtypes = [C.c_void_p, C.c_uint64, C.c_char_p, C.c_int]
+        for f, rt in (("header", C.c_void_p), ("data", C.c_void_p), ("size", C.c_uint64), ("first_record", C.c_uint64), ("first_line", C.c_int64)):
+            fn = getattr(L, "bkid_host_sam_" + f)
+            fn.restype = rt
+            fn.argtypes = [C.c_void_p]
+        L.bkid_host_sam_close.argtypes = [C.c_void_p]
         _host = L
     return _host
 
@@ -280,7 +289,7 @@ EXPORTS = ["bkid_abi_version", "bkid_last_error", "bkid_default_params", "bkid_c
            "bkid_shard_finish", "bkid_fetch_bucket_ranks", "bkid_device_copy",
            "bkid_push_bgzf", "bkid_push_bgzf_range", "bkid_get_decode_stats", "bkid_fetch_column", "bkid_set_exclude", "bkid_device_gather_rows", "bkid_op_banded_align", "bkid_profile_kernels", "bkid_profile_report",
            "bkid_comm_nccl_unique_id", "bkid_comm_nccl_init", "bkid_comm_nccl_init_all", "bkid_comm_local_create", "bkid_comm_destroy", "bkid_dist_run", "bkid_dist_run_threads",
-           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table", "bkid_sort_records"]
+           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table", "bkid_sort_records", "bkid_push_sam"]
 
 CAND_BYTES = 48
 SAROW_BYTES = 88
@@ -311,6 +320,7 @@ def cuda_lib():
         L.bkid_push_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_int64, C.c_uint64, C.POINTER(C.c_int64)]
         L.bkid_push_bgzf_range.argtypes = [vp, vp, C.c_uint64, vp, C.c_int64, C.c_uint64, C.c_int64, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.bkid_get_decode_stats.argtypes = [vp, C.POINTER(DecodeStats)]
+        L.bkid_push_sam.argtypes = [vp, vp, C.c_uint64, C.c_int64, C.POINTER(C.c_int64)]
         L.bkid_fetch_column.argtypes = [vp, C.c_char_p, vp, C.c_int64, C.POINTER(C.c_int64)]
         L.bkid_reset.argtypes = [vp]
         L.bkid_sort_records.argtypes = [vp, C.POINTER(C.c_int32)]
@@ -461,6 +471,45 @@ class BgzfFile:
             pass
 
 
+class SamFile:
+    """Host half of the SAM path: mapped SAM file (or a header in a caller's buffer) + the target table of its @SQ
+    lines (``bkid_host_sam_open`` / ``bkid_host_sam_parse``, breakid_b200/host/bam_reader.h).  ``text`` is a view of the
+    alignment lines, which start on file line ``first_line``."""
+
+    def __init__(self, path: Optional[str] = None, buf: Optional[bytes] = None):
+        self.lib = host_lib()
+        err = C.create_string_buffer(256)
+        self._buf = None
+        if buf is not None:
+            self._buf = C.create_string_buffer(bytes(buf), len(buf))
+            self.h = self.lib.bkid_host_sam_parse(C.cast(self._buf, C.c_void_p), len(buf), err, 256)
+        else:
+            self.h = self.lib.bkid_host_sam_open(path.encode(), err, 256)
+        if not self.h:
+            raise IOError("SAM header: " + err.value.decode())
+        hd = C.cast(self.lib.bkid_host_sam_header(self.h), C.POINTER(Header)).contents
+        self.target_len = [int(hd.target_len[i]) for i in range(hd.n_targets)]
+        self.target_names = [hd.target_name[i].decode() for i in range(hd.n_targets)]
+        self.data = self.lib.bkid_host_sam_data(self.h)
+        self.size = int(self.lib.bkid_host_sam_size(self.h))
+        self.first_record = int(self.lib.bkid_host_sam_first_record(self.h))
+        self.first_line = int(self.lib.bkid_host_sam_first_line(self.h))
+
+    def text(self) -> bytes:
+        return C.string_at(self.data + self.first_record, self.size - self.first_record) if self.size > self.first_record else b""
+
+    def close(self):
+        if self.h:
+            self.lib.bkid_host_sam_close(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Context:
     """One device context (``bkid_ctx``)."""
 
@@ -529,6 +578,21 @@ class Context:
         self._chk(self.lib.bkid_push_bgzf_range(self.ctx, C.c_void_p(data_ptr if data_ptr is not None else f.data), f.size, C.c_void_p(f.blocks), f.n_blocks,
                                                 f.first_record, first_block, end_block, C.byref(n), C.byref(a), C.byref(b)))
         return int(n.value), int(a.value), int(b.value)
+
+    def push_sam(self, text, first_line: int = 1, data_ptr=None, size=None) -> int:
+        """device parse of SAM alignment lines (``bkid_push_sam``); returns the record count.  ``text`` is bytes (its
+        lines start on file line ``first_line``) or a ``SamFile`` (its alignment lines, numbered from the file).
+        ``data_ptr`` / ``size`` push that host memory instead (e.g. a pinned copy of the text)."""
+        n = C.c_int64()
+        if isinstance(text, SamFile):
+            ptr, ln, first_line = text.data + text.first_record, text.size - text.first_record, text.first_line
+            keep = text
+        else:
+            keep = C.create_string_buffer(bytes(text), len(text)) if data_ptr is None else None
+            ptr, ln = (C.cast(keep, C.c_void_p).value, len(text)) if data_ptr is None else (data_ptr, size)
+        self._chk(self.lib.bkid_push_sam(self.ctx, C.c_void_p(ptr), ln, first_line, C.byref(n)))
+        del keep
+        return int(n.value)
 
     def decode_stats(self) -> dict:
         s = DecodeStats()

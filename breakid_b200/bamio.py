@@ -1,4 +1,4 @@
-"""Minimal BAM *writer* for synthetic workloads (test / bench tooling, not on the hot path).
+"""Minimal BAM / SAM *writer* for synthetic workloads (test / bench tooling, not on the hot path).
 
 Writes the record batch of ``synth.SynthData`` in its own record order as a real BGZF-compressed BAM so
 that the unmodified reference CPU binary can be run on byte-identical input.  ``sort_order`` is the @HD SO: tag
@@ -153,20 +153,75 @@ def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: in
     out.close()
 
 
+_NT16 = np.frombuffer(b"=ACMGRSVTWYHKDBN", dtype=np.uint8)
+
+
+def write_sam(path: str, d: synth.SynthData, random_qual: bool = True, chunk: int = 200_000, sa_seq=None,
+              sort_order: str = "coordinate") -> None:
+    """The records ``write_bam`` writes (same arguments, same names, cigars, SA tags, bases and qualities) as SAM text:
+    RNEXT is "=" when the mate is on the record's own target, SEQ spells the 4-bit codes, QUAL is Phred + 33."""
+    cfg = d.cfg
+    L = cfg.read_len
+    c = {k: v.cpu().numpy() for k, v in d.cols.items()}
+    n = c["flag"].shape[0]
+    sa_rec = d.sa_rec.cpu().numpy()
+    cig_off = d.cig_off.cpu().numpy(); cig_ops = d.cig_ops.cpu().numpy().astype(np.uint32)
+    sa_off = d.sa_off.cpu().numpy(); sa_txt = d.sa_txt.cpu().numpy()
+    sa_slot = np.full(n, -1, dtype=np.int64); sa_slot[sa_rec] = np.arange(sa_rec.shape[0])
+    rng = np.random.RandomState(cfg.seed + 12345)          # the qualities write_bam draws, in the same order
+    names = [synth.chrom_name(t) for t in range(len(cfg.chrom_lens))]
+    with open(path, "wb") as out:
+        out.write(("@HD\tVN:1.4\tSO:%s\n" % sort_order + "".join("@SQ\tSN:%s\tLN:%d\n" % (names[t], l) for t, l in enumerate(cfg.chrom_lens))).encode())
+        plain = "%dM" % L
+        seq_plain = b"A" * L
+        for s in range(0, n, chunk):
+            e = min(n, s + chunk)
+            m = e - s
+            q = (rng.randint(2, 41, (m, L)).astype(np.uint8) if random_qual else np.full((m, L), 30, np.uint8)) + 33
+            qb = q.tobytes()
+            tid = c["tid"][s:e].tolist(); pos = c["pos"][s:e].tolist(); mapq = c["mapq"][s:e].tolist(); flag = c["flag"][s:e].tolist()
+            mtid = c["mtid"][s:e].tolist(); mpos = c["mpos"][s:e].tolist(); isize = c["isize"][s:e].tolist(); nid = c["name_id"][s:e].tolist()
+            parts = []
+            for j in range(m):
+                t, mt = tid[j], mtid[j]
+                k = sa_slot[s + j]
+                rn = names[t] if t >= 0 else "*"
+                rx = "*" if mt < 0 else "=" if mt == t else names[mt]
+                if k < 0:
+                    parts.append(("r%010d\t%d\t%s\t%d\t%d\t%s\t%s\t%d\t%d\t" % (nid[j], flag[j], rn, pos[j] + 1, mapq[j], plain, rx, mpos[j] + 1, isize[j])).encode())
+                    parts.append(seq_plain); parts.append(b"\t"); parts.append(qb[j * L:(j + 1) * L]); parts.append(b"\n")
+                    continue
+                ops = cig_ops[cig_off[k]:cig_off[k + 1]]
+                cig = "".join("%d%s" % (int(o) >> 4, "MIDNSHP=X"[int(o) & 15]) for o in ops)
+                if sa_seq is None:
+                    sq = seq_plain
+                else:
+                    b = np.asarray(sa_seq["seq4"][int(sa_seq["seq_off"][k]):int(sa_seq["seq_off"][k + 1])], np.uint8)
+                    sq = _NT16[np.stack([b >> 4, b & 15], 1).reshape(-1)[:L]].tobytes()
+                parts.append(("r%010d\t%d\t%s\t%d\t%d\t%s\t%s\t%d\t%d\t" % (nid[j], flag[j], rn, pos[j] + 1, mapq[j], cig, rx, mpos[j] + 1, isize[j])).encode())
+                parts.append(sq); parts.append(b"\t" + b"?" * L + b"\tSA:Z:"); parts.append(sa_txt[sa_off[k]:sa_off[k + 1]].tobytes()); parts.append(b"\n")
+            out.write(b"".join(parts))
+
+
 def write_dataset(dirpath: str, d: synth.SynthData, random_qual: bool = True, nib: bool = True,
-                  genes_per_mb: float = 4.0, sort_order: str = "coordinate") -> dict:
+                  genes_per_mb: float = 4.0, sort_order: str = "coordinate", sam: bool = False) -> dict:
     """Lay down everything a BreakID run needs: <dir>/reads.bam, <dir>/nib/{ref_names.txt,
-    hg19_<chr>.nib}, <dir>/ref_files/refGene.txt.  Returns the paths."""
+    hg19_<chr>.nib}, <dir>/ref_files/refGene.txt, and with ``sam`` also <dir>/reads.sam (the same records as text).
+    Returns the paths."""
     import os
     os.makedirs(os.path.join(dirpath, "nib"), exist_ok=True)
     os.makedirs(os.path.join(dirpath, "ref_files"), exist_ok=True)
     cfg = d.cfg
     bam = os.path.join(dirpath, "reads.bam")
     write_bam(bam, d, random_qual=random_qual, sort_order=sort_order)
+    paths = {}
+    if sam:
+        paths["sam"] = os.path.join(dirpath, "reads.sam")
+        write_sam(paths["sam"], d, random_qual=random_qual, sort_order=sort_order)
     synth.write_ref_names(os.path.join(dirpath, "nib", "ref_names.txt"), len(cfg.chrom_lens))
     if nib:
         for t, l in enumerate(cfg.chrom_lens):
             pay = synth.random_nib_bytes(l, cfg.seed * 1000 + t)
             synth.write_nib(os.path.join(dirpath, "nib", "hg19_%s.nib" % synth.chrom_name(t)), pay, l)
     synth.write_refgene(os.path.join(dirpath, "ref_files", "refGene.txt"), cfg.chrom_lens, genes_per_mb=genes_per_mb)
-    return {"bam": bam, "nib": os.path.join(dirpath, "nib"), "refgene": os.path.join(dirpath, "ref_files", "refGene.txt")}
+    return dict({"bam": bam, "nib": os.path.join(dirpath, "nib"), "refgene": os.path.join(dirpath, "ref_files", "refGene.txt")}, **paths)

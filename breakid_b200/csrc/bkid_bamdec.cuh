@@ -350,6 +350,8 @@ struct bkid_decoder {                 // per-context streaming state, allocated 
   bamdec::Task *h_tasks = nullptr; size_t h_tasks_cap = 0;
   cudaStream_t st_copy = nullptr;
   cudaEvent_t ev_h2d[2], ev_free[2], ev_t[8];
+  DBuf aux, nm_txt, nm_off, nm_slot;    // SAM decode (bkid_samdec.cuh): per-line fields, target-name lookup table
+  uint32_t nm_mask = 0; bool names_built = false;
   bool init = false;
   bool skip_crc = false;                // BKID_BGZF_NO_CRC=1: timing experiments only
   bkid_decode_stats stats;
@@ -372,7 +374,7 @@ static void decoder_free(bkid_ctx *c)
 {
   bkid_decoder *d = c->dec;
   if (!d) return;
-  for (DBuf *b : {&d->comp[0], &d->comp[1], &d->unc, &d->carry, &d->tasks, &d->seed, &d->cnt, &d->land, &d->base, &d->rec_off, &d->state}) b->release();
+  for (DBuf *b : {&d->comp[0], &d->comp[1], &d->unc, &d->carry, &d->tasks, &d->seed, &d->cnt, &d->land, &d->base, &d->rec_off, &d->state, &d->aux, &d->nm_txt, &d->nm_off, &d->nm_slot}) b->release();
   for (auto &b : d->meta) b.release();
   for (auto &b : d->metao) b.release();
   for (int i = 0; i < 2; ++i) if (d->h_stage[i]) cudaFreeHost(d->h_stage[i]);

@@ -1496,4 +1496,5 @@ __global__ void pair_xy(const bkid_pair *__restrict__ pairs, long long np, uint3
 #include "bkid_sort.cuh"
 #include "bkid_dist.cuh"
 #include "bkid_bamdec.cuh"
+#include "bkid_samdec.cuh"
 #include "bkid_align_api.cuh"

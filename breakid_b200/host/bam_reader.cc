@@ -426,3 +426,98 @@ extern "C" uint64_t bkid_host_bgzf_first_record(const bkid_host_bgzf *h) { retur
 extern "C" uint64_t bkid_host_bgzf_usize(const bkid_host_bgzf *h) { return h->usize; }
 extern "C" int32_t bkid_host_bgzf_first_l_qseq(const bkid_host_bgzf *h) { return h->first_l_qseq; }
 extern "C" void bkid_host_bgzf_close(bkid_host_bgzf *h) { if (!h) return; munmap((void *)h->file, h->fsz); delete h; }
+
+// ---- host half of the SAM path (bkid_push_sam): the @SQ lines of the header become the target table ----------
+struct bkid_host_sam {
+  const uint8_t *data = nullptr; size_t size = 0;
+  bool mapped = false;
+  std::vector<uint32_t> target_len;
+  std::vector<std::string> names;
+  std::vector<const char *> name_ptrs;
+  bkid_header hdr;
+  uint64_t first_record = 0;
+  int64_t first_line = 1;
+};
+
+static bool sam_parse_header(bkid_host_sam *h, std::string &msg)
+{
+  const char *p = (const char *)h->data, *end = p + h->size;
+  int64_t line = 1;
+  std::vector<std::string> seen;
+  while (p < end && *p == '@') {
+    const char *nl = (const char *)memchr(p, '\n', (size_t)(end - p));
+    const char *le = nl ? nl : end;
+    std::string ln(p, (size_t)(le - p));
+    if (!ln.empty() && ln.back() == '\r') ln.pop_back();
+    if (ln.compare(0, 4, "@SQ\t") == 0) {
+      std::string sn, lnv;
+      bool have_sn = false, have_ln = false;
+      for (size_t a = 4; a <= ln.size();) {
+        size_t b = ln.find('\t', a);
+        if (b == std::string::npos) b = ln.size();
+        std::string f = ln.substr(a, b - a);
+        if (f.compare(0, 3, "SN:") == 0 && !have_sn) { sn = f.substr(3); have_sn = true; }
+        if (f.compare(0, 3, "LN:") == 0 && !have_ln) { lnv = f.substr(3); have_ln = true; }
+        a = b + 1;
+      }
+      const std::string where = "header line " + std::to_string(line) + ": ";
+      if (!have_sn || sn.empty()) { msg = where + "@SQ without SN"; return false; }
+      if (!have_ln) { msg = where + "@SQ " + sn + " without LN"; return false; }
+      unsigned long long v = 0;
+      bool ok = !lnv.empty() && lnv.size() <= 10;
+      for (char ch : lnv) { ok = ok && ch >= '0' && ch <= '9'; v = v * 10 + (unsigned)(ch - '0'); }
+      if (!ok || v > 0x7fffffffull) { msg = where + "LN of " + sn + " is not a number in 0..2^31-1"; return false; }
+      for (const std::string &s : h->names)
+        if (s == sn) { msg = where + "duplicate @SQ SN " + sn; return false; }
+      h->names.push_back(sn);
+      h->target_len.push_back((uint32_t)v);
+    }
+    ++line;
+    p = nl ? nl + 1 : end;
+  }
+  h->first_record = (uint64_t)(p - (const char *)h->data);
+  h->first_line = line;
+  for (auto &s : h->names) h->name_ptrs.push_back(s.c_str());
+  h->hdr.n_targets = (int32_t)h->names.size();
+  h->hdr.target_len = h->target_len.data();
+  h->hdr.target_name = h->name_ptrs.data();
+  return true;
+}
+
+extern "C" bkid_host_sam *bkid_host_sam_open(const char *path, char *err, int errlen)
+{
+  int fd = open(path, O_RDONLY);
+  if (fd < 0) { set_err(err, errlen, std::string("cannot open ") + path); return nullptr; }
+  struct stat st;
+  if (fstat(fd, &st) != 0 || st.st_size <= 0) { close(fd); set_err(err, errlen, std::string("cannot stat ") + path + " (or it is empty)"); return nullptr; }
+  size_t fsz = (size_t)st.st_size;
+  const uint8_t *file = (const uint8_t *)mmap(nullptr, fsz, PROT_READ, MAP_PRIVATE, fd, 0);
+  close(fd);
+  if (file == MAP_FAILED) { set_err(err, errlen, "mmap failed"); return nullptr; }
+  bkid_host_sam *h = new bkid_host_sam();
+  h->data = file; h->size = fsz; h->mapped = true;
+  std::string msg;
+  if (!sam_parse_header(h, msg)) { set_err(err, errlen, msg.c_str()); munmap((void *)file, fsz); delete h; return nullptr; }
+  return h;
+}
+
+extern "C" bkid_host_sam *bkid_host_sam_parse(const uint8_t *buf, uint64_t len, char *err, int errlen)
+{
+  bkid_host_sam *h = new bkid_host_sam();
+  h->data = buf; h->size = (size_t)len;
+  std::string msg;
+  if (!sam_parse_header(h, msg)) { set_err(err, errlen, msg.c_str()); delete h; return nullptr; }
+  return h;
+}
+
+extern "C" const bkid_header *bkid_host_sam_header(const bkid_host_sam *h) { return &h->hdr; }
+extern "C" const uint8_t *bkid_host_sam_data(const bkid_host_sam *h) { return h->data; }
+extern "C" uint64_t bkid_host_sam_size(const bkid_host_sam *h) { return h->size; }
+extern "C" uint64_t bkid_host_sam_first_record(const bkid_host_sam *h) { return h->first_record; }
+extern "C" int64_t bkid_host_sam_first_line(const bkid_host_sam *h) { return h->first_line; }
+extern "C" void bkid_host_sam_close(bkid_host_sam *h)
+{
+  if (!h) return;
+  if (h->mapped) munmap((void *)h->data, h->size);
+  delete h;
+}

@@ -31,6 +31,21 @@ uint64_t bkid_host_bgzf_usize(const bkid_host_bgzf *h);                 /* total
 int32_t bkid_host_bgzf_first_l_qseq(const bkid_host_bgzf *h);           /* read length of the first record (driver's _params.txt), -1 if none */
 void bkid_host_bgzf_close(bkid_host_bgzf *h);
 
+/* Host half of the SAM path (bkid_push_sam): the header's @SQ SN:/LN: lines become the target table in @SQ order
+ * (other header lines are ignored; a duplicate SN, an @SQ without SN, or a missing or non-numeric LN is an error).
+ * The alignment lines start at first_record, on file line first_line (1-based).  A file without header lines is valid
+ * (it has no targets: every RNAME must be *).  bkid_host_sam_open maps a file; bkid_host_sam_parse reads the header
+ * lines at the start of a caller-owned buffer (e.g. what was read from stdin) and keeps pointing into it. */
+typedef struct bkid_host_sam bkid_host_sam;
+bkid_host_sam *bkid_host_sam_open(const char *path, char *err, int errlen);
+bkid_host_sam *bkid_host_sam_parse(const uint8_t *buf, uint64_t len, char *err, int errlen);
+const bkid_header *bkid_host_sam_header(const bkid_host_sam *h);
+const uint8_t *bkid_host_sam_data(const bkid_host_sam *h);              /* the mapped file / the buffer */
+uint64_t bkid_host_sam_size(const bkid_host_sam *h);
+uint64_t bkid_host_sam_first_record(const bkid_host_sam *h);            /* offset of the first alignment line */
+int64_t bkid_host_sam_first_line(const bkid_host_sam *h);               /* its 1-based line number */
+void bkid_host_sam_close(bkid_host_sam *h);
+
 #ifdef __cplusplus
 }
 #endif

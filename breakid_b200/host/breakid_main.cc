@@ -13,8 +13,12 @@
 //     ranks are NCCL calls inside the library (bkid_dist_run).  A device may be named more than once (-gpu 0,0,0): the
 //     ranks then share it and exchange through device copies -- that is how the path is tested on a one-GPU box;
 //   * -sort  the BAM may be in any record order (e.g. read-name grouped, as bwa mem | samblaster writes it): the records are
-//     coordinate sorted on the device after decode (bkid_sort_records), and no .bai is required.  One GPU only.
-// Host work: BAM decode (bam_reader.cc), .nib loading, refGene annotation, the final unstable sort
+//     coordinate sorted on the device after decode (bkid_sort_records), and no .bai is required.  One GPU only;
+//   * -i may name SAM text instead of a BAM (a file whose first line is a header line or an alignment line of 11 or more
+//     tab-separated fields), or be - to read SAM from stdin: the lines are parsed on the device (bkid_push_sam), and no
+//     .bai is required.  A BAM (first bytes 1f 8b) takes the BAM path unchanged.  With -gpu a,b,... every rank parses
+//     the newline-aligned byte range of a coordinate-sorted SAM file that falls to it; stdin needs one GPU.
+// Host work: BAM / SAM header parsing (bam_reader.cc), .nib loading, refGene annotation, the final unstable sort
 // by N_DRP and file writing.  Everything between decode and the cluster records runs on the GPU.
 #include <getopt.h>
 #include <sys/stat.h>
@@ -41,7 +45,7 @@ static const char *kHelp =
     " Usage: \n \t BreakID -i input.bam -o prefix -n nib_folder <options> \n\n "
     "     DESCRIPTION\n "
     "     \t -h -? -help \t help\n "
-    "     \t -i*        \t input bam-file\n "
+    "     \t -i*        \t input bam-file, or SAM text (a file, or - for stdin)\n "
     "     \t -o*        \t output file (prefix only)\n "
     "     \t -n*        \t folder name to nib files\n "
     "     \t -q         \t encompassing reads quality thresholds  [20]\n"
@@ -65,6 +69,21 @@ struct CallRow {
 
 static bool exists(const std::string &p) { struct stat st; return stat(p.c_str(), &st) == 0; }
 static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+// 0 = BAM (gzip magic), 1 = SAM (the first line is a header line or has at least 11 tab-separated fields), -1 = neither
+static int sniff_input(const std::string &path)
+{
+  FILE *f = fopen(path.c_str(), "rb");
+  if (!f) return -1;
+  std::string b(65536, '\0');
+  b.resize(fread(&b[0], 1, b.size(), f));
+  fclose(f);
+  if (b.size() >= 2 && (uint8_t)b[0] == 0x1f && (uint8_t)b[1] == 0x8b) return 0;
+  if (b.empty()) return -1;
+  if (b[0] == '@') return 1;
+  std::string first = b.substr(0, b.find('\n'));
+  return std::count(first.begin(), first.end(), '\t') >= 10 ? 1 : -1;
+}
 
 static bool cmp_cluster(const CallRow &a, const CallRow &b) { return a.c.n_discordant_pair > b.c.n_discordant_pair; }   // reference src/BreakID.h:185-188
 
@@ -222,8 +241,39 @@ int main(int argc, char *argv[])
   const bool host_decode = getenv("BKID_HOST_DECODE") && atoi(getenv("BKID_HOST_DECODE")) != 0;
   bkid_host_bam *bam = nullptr;
   bkid_host_bgzf *bgzf = nullptr;
+  bkid_host_sam *sam = nullptr;
   const bkid_header *hdr = nullptr;
-  if (host_decode) {
+  const bool from_stdin = inp == "-";
+  const bool is_sam = from_stdin || sniff_input(inp) == 1;
+  std::vector<uint8_t> sbuf;                           // stdin: the text read so far and not yet pushed
+  size_t spos = 0;                                     // stdin: start of the unpushed text in sbuf
+  bool seof = false;
+  const size_t PIECE = (size_t)256 << 20;
+  auto sfill = [&]() {
+    size_t o = sbuf.size();
+    sbuf.resize(o + PIECE);
+    size_t n = fread(sbuf.data() + o, 1, PIECE, stdin);
+    sbuf.resize(o + n);
+    if (n == 0) seof = true;
+  };
+  if (is_sam && host_decode) { std::cerr << "Error: host decode reads BAM only (unset BKID_HOST_DECODE for SAM input)\n"; exit(1); }
+  if (from_stdin && gpus.size() > 1) { std::cerr << "Error: SAM from stdin needs one GPU; give a SAM file to use several (-gpu " << gpus.size() << " devices)\n"; exit(1); }
+  if (from_stdin) {
+    for (;;) {                                         // the header lines come first
+      if (spos >= sbuf.size()) { if (seof) break; sfill(); continue; }
+      if (sbuf[spos] != '@') break;
+      const void *nl = memchr(sbuf.data() + spos, '\n', sbuf.size() - spos);
+      if (!nl) { if (seof) { spos = sbuf.size(); break; } sfill(); continue; }
+      spos = (size_t)((const uint8_t *)nl - sbuf.data()) + 1;
+    }
+    sam = bkid_host_sam_parse(sbuf.data(), spos, err, sizeof err);
+    if (!sam) { std::cerr << "Error: can not read sam header from stdin: " << err << std::endl; exit(1); }
+    hdr = bkid_host_sam_header(sam);
+  } else if (is_sam) {
+    sam = bkid_host_sam_open(inp.c_str(), err, sizeof err);
+    if (!sam) { std::cerr << "Error: can not open sam-file: " << inp << " (" << err << ")" << std::endl; exit(1); }
+    hdr = bkid_host_sam_header(sam);
+  } else if (host_decode) {
     bam = bkid_host_read_bam(inp.c_str(), threads, err, sizeof err);
     if (!bam) { std::cerr << "Error: can not open bam-file: " << inp << std::endl; exit(1); }
     hdr = bkid_host_bam_header(bam);
@@ -268,10 +318,38 @@ int main(int argc, char *argv[])
       if (!xt.empty() && bkid_set_exclude(ctxs[r], (int64_t)xt.size(), xt.data(), xb.data(), xe.data())) { std::cerr << "Error: set_exclude: " << bkid_last_error(ctxs[r]) << std::endl; exit(1); }
     }
     double t_push0 = now_s();
-    const int64_t nblk = bkid_host_bgzf_n_blocks(bgzf);
     std::vector<int64_t> nrec(W, 0);
     std::vector<uint64_t> first(W, 0), next(W, 0);
     std::vector<int> rcs(W, 0);
+    if (sam) {
+      // rank r parses the newline-aligned byte range [cut_r, cut_r+1): cut_r is the first line start at or after r * size / W
+      const uint8_t *text = bkid_host_sam_data(sam);
+      const uint64_t size = bkid_host_sam_size(sam), f0 = bkid_host_sam_first_record(sam);
+      std::vector<uint64_t> cut(W + 1, size);
+      cut[0] = f0;
+      for (int r = 1; r < W; ++r) {
+        uint64_t p = std::max<uint64_t>(f0, size * (uint64_t)r / (uint64_t)W);
+        if (p > f0 && p < size && text[p - 1] != '\n') {
+          const void *nl = memchr(text + p, '\n', (size_t)(size - p));
+          p = nl ? (uint64_t)((const uint8_t *)nl - text) + 1 : size;
+        }
+        cut[r] = std::max(p, cut[r - 1]);
+      }
+      std::vector<int64_t> lines(W + 1, bkid_host_sam_first_line(sam));     // file line number of every cut (error messages)
+      {
+        std::vector<std::thread> th;
+        for (int r = 0; r < W; ++r) th.emplace_back([&, r] { lines[r + 1] = std::count(text + cut[r], text + cut[r + 1], '\n'); });
+        for (auto &t : th) t.join();
+        for (int r = 0; r < W; ++r) lines[r + 1] += lines[r];
+      }
+      std::vector<std::thread> th;
+      for (int r = 0; r < W; ++r)
+        th.emplace_back([&, r] { rcs[r] = bkid_push_sam(ctxs[r], text + cut[r], cut[r + 1] - cut[r], lines[r], &nrec[r]); });
+      for (auto &t : th) t.join();
+      for (int r = 0; r < W; ++r)
+        if (rcs[r]) { std::cerr << "Error: can not read sam-file: " << inp << " (" << bkid_last_error(ctxs[r]) << ")" << std::endl; exit(1); }
+    } else {
+    const int64_t nblk = bkid_host_bgzf_n_blocks(bgzf);
     {
       std::vector<std::thread> th;
       for (int r = 0; r < W; ++r)
@@ -285,6 +363,7 @@ int main(int argc, char *argv[])
       if (rcs[r]) { std::cerr << "Error: can not read bam-file: " << inp << " (" << bkid_last_error(ctxs[r]) << ")" << std::endl; exit(1); }
     for (int r = 0; r + 1 < W; ++r)        // where one range landed is where the next one started: the union is exactly the file's record sequence
       if (next[r] != first[r + 1]) { std::cerr << "Error: can not read bam-file: " << inp << " (the block ranges of ranks " << r << " and " << r + 1 << " do not stitch)" << std::endl; exit(1); }
+    }
     double t_push = now_s() - t_push0;
     // nib files are needed by the refinement of every rank (41-mers are replicated work)
     for (int t = 0; t < hdr->n_targets; ++t) {
@@ -316,11 +395,12 @@ int main(int argc, char *argv[])
     cl.resize((size_t)n);
     int64_t pairs = 0, masked = 0, clustered = 0, nclusters = 0, records = 0;
     for (int r = 0; r < W; ++r) { bkid_timings t; bkid_get_timings(ctxs[r], &t); pairs += t.n_pairs; masked += t.n_masked; clustered += t.n_clustered; nclusters += t.n_clusters; records += nrec[r]; }
-    finish_and_write(inp, out, refgene, names, cl, filter, true, qual, dist[0], clustered > 0, t_start, pairs, masked, clustered, nclusters, t_run, 0.0, 0.0,
-                     [&](std::ofstream &j) { j << "decoder\tdevice\nranks\t" << W << "\ncommunicator\t" << (distinct ? "nccl" : "local") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push
+    finish_and_write(inp, out, refgene, names, cl, filter, !sam, qual, dist[0], clustered > 0, t_start, pairs, masked, clustered, nclusters, t_run, 0.0, 0.0,
+                     [&](std::ofstream &j) { j << "decoder\t" << (sam ? "sam" : "device") << "\nranks\t" << W << "\ncommunicator\t" << (distinct ? "nccl" : "local") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push
                                                 << "\nrun_s\t" << t_run << "\nrecords\t" << records << "\n"; });
     for (int r = 0; r < W; ++r) { bkid_comm_destroy(comms[r]); bkid_destroy(ctxs[r]); }
-    bkid_host_bgzf_close(bgzf);
+    if (bgzf) bkid_host_bgzf_close(bgzf);
+    if (sam) bkid_host_sam_close(sam);
     return 0;
   }
   bkid_ctx *ctx = bkid_create(gpu, hdr, &prm);
@@ -332,6 +412,38 @@ int main(int argc, char *argv[])
   memset(&dst, 0, sizeof dst);
   if (host_decode) {
     if (bkid_push_batch(ctx, bkid_host_bam_batch_narrow(bam))) die("push_batch");
+  } else if (sam) {
+    auto push = [&](const uint8_t *text, uint64_t len, int64_t line) -> int64_t {
+      int64_t nrec = 0;
+      if (bkid_push_sam(ctx, text, len, line, &nrec)) {
+        std::cerr << "Error: can not read sam-file: " << inp << " (" << bkid_last_error(ctx) << ")" << std::endl;
+        exit(1);
+      }
+      bkid_decode_stats s;
+      bkid_get_decode_stats(ctx, &s);
+      dst.n_chunks += s.n_chunks; dst.uncompressed_bytes += s.uncompressed_bytes; dst.n_records += s.n_records;
+      dst.total_ms += s.total_ms; dst.boundaries_ms += s.boundaries_ms; dst.extract_ms += s.extract_ms;
+      return nrec;
+    };
+    int64_t line = bkid_host_sam_first_line(sam);
+    if (!from_stdin) {
+      const uint64_t f0 = bkid_host_sam_first_record(sam);
+      push(bkid_host_sam_data(sam) + f0, bkid_host_sam_size(sam) - f0, line);
+    } else {
+      for (;;) {                                       // each call gets the complete lines read so far; a partial last line waits
+        const bool last = seof;
+        size_t end = sbuf.size();
+        if (!last) {
+          const void *nl = spos < sbuf.size() ? memrchr(sbuf.data() + spos, '\n', sbuf.size() - spos) : nullptr;
+          end = nl ? (size_t)((const uint8_t *)nl - sbuf.data()) + 1 : spos;
+        }
+        if (end > spos) line += push(sbuf.data() + spos, end - spos, line);
+        if (last) break;
+        sbuf.erase(sbuf.begin(), sbuf.begin() + end);
+        spos = 0;
+        sfill();
+      }
+    }
   } else {
     int64_t nrec = 0;
     if (bkid_push_bgzf(ctx, bkid_host_bgzf_data(bgzf), bkid_host_bgzf_size(bgzf), bkid_host_bgzf_blocks(bgzf), bkid_host_bgzf_n_blocks(bgzf), bkid_host_bgzf_first_record(bgzf), &nrec)) {
@@ -367,7 +479,7 @@ int main(int argc, char *argv[])
   std::vector<bkid_cluster_rec> cl;
   double t_bp = 0;
   if (tm.n_clustered > 0) {
-    if (!sort && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
+    if (!sort && !sam && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
       std::cerr << "Error: please index bam-file first:\t" << inp << std::endl;                     // src/BreakID.cc:412-416
       exit(1);
     }
@@ -385,10 +497,15 @@ int main(int argc, char *argv[])
     cl.resize((size_t)n);
   }
   bkid_get_timings(ctx, &tm);
-  finish_and_write(inp, out, refgene, names, cl, filter, !sort, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
+  finish_and_write(inp, out, refgene, names, cl, filter, !sort && !sam, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
                    [&](std::ofstream &j) {
-                     j << "decoder\t" << (host_decode ? "host" : "device") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ninflate_ms\t" << dst.inflate_ms << "\nboundaries_ms\t" << dst.boundaries_ms
-                       << "\nextract_ms\t" << dst.extract_ms << "\ncompressed_bytes\t" << dst.compressed_bytes << "\nuncompressed_bytes\t" << dst.uncompressed_bytes << "\nrecords\t" << tm.n_records << "\nh2d_ms\t" << tm.h2d << "\nclassify_ms\t" << tm.classify << "\ninsert_stats_ms\t" << tm.insert_stats
+                     if (sam)
+                       j << "decoder\tsam\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ntext_bytes\t" << dst.uncompressed_bytes << "\nlines_ms\t" << dst.boundaries_ms << "\nparse_ms\t" << dst.extract_ms
+                         << "\nsam_chunks\t" << dst.n_chunks;
+                     else
+                       j << "decoder\t" << (host_decode ? "host" : "device") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ninflate_ms\t" << dst.inflate_ms << "\nboundaries_ms\t" << dst.boundaries_ms
+                         << "\nextract_ms\t" << dst.extract_ms << "\ncompressed_bytes\t" << dst.compressed_bytes << "\nuncompressed_bytes\t" << dst.uncompressed_bytes;
+                     j << "\nrecords\t" << tm.n_records << "\nh2d_ms\t" << tm.h2d << "\nclassify_ms\t" << tm.classify << "\ninsert_stats_ms\t" << tm.insert_stats
                        << "\njoin_ms\t" << tm.join << "\nbucket_sort_ms\t" << tm.bucket_sort << "\nmask_ms\t" << tm.mask << "\ncluster_ms\t" << tm.cluster << "\nsummarize_ms\t" << tm.summarize
                        << "\nevidence_ms\t" << tm.evidence << "\nrefine_ms\t" << tm.refine << "\n";
                      if (sort) j << "sort_ms\t" << t_sort * 1e3 << "\ninput_was_sorted\t" << was_sorted << "\n";
@@ -396,5 +513,6 @@ int main(int argc, char *argv[])
   bkid_destroy(ctx);
   if (bam) bkid_host_bam_free(bam);
   if (bgzf) bkid_host_bgzf_close(bgzf);
+  if (sam) bkid_host_sam_close(sam);
   return 0;
 }

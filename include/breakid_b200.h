@@ -224,6 +224,19 @@ int bkid_push_bgzf_range(bkid_ctx *ctx, const uint8_t *file, uint64_t file_size,
                          uint64_t first_record_uoffset, int64_t first_block, int64_t end_block, int64_t *n_records,
                          uint64_t *first_record_uoff, uint64_t *next_record_uoff);
 int bkid_get_decode_stats(bkid_ctx *ctx, bkid_decode_stats *stats);
+/* Extension (the reference reads BAM only): append the records of SAM alignment text, parsed on the device.
+ * `text` holds alignment lines only (no header), in host memory (pinned memory is copied from directly, pageable memory
+ * through the library's pinned staging); it ends at a line end or at the end of a complete last line.  Every column
+ * bkid_fetch_column returns is byte-identical to what bkid_push_bgzf leaves for a BAM holding the same records (SAM spec
+ * 1.4 / 4.2): RNAME / RNEXT resolve against the context's target names in header order ("*" -> -1, RNEXT "=" -> the
+ * record's own tid), POS / PNEXT are 1-based, SEQ letters become BAM 4-bit codes, the first SA:Z / OC:Z fields give the
+ * SA / OC text.  Each line needs at least 11 tab-separated fields; a \r before the newline is dropped.  Anything else
+ * (empty or '@' lines, numbers out of range, unknown reference names, bad CIGAR, SEQ / QUAL / CIGAR lengths that
+ * disagree, optional fields that are not TG:T:VALUE of type AifZHB) returns BKID_ERR_IO with a message naming the file
+ * line (`first_line` = 1-based line number of text[0]) and the field; the context then holds exactly what it held
+ * before the call.  bkid_get_decode_stats: uncompressed_bytes = text bytes, boundaries_ms = line split, extract_ms =
+ * parse; inflate_ms and compressed_bytes are 0. */
+int bkid_push_sam(bkid_ctx *ctx, const uint8_t *text, uint64_t len, int64_t first_line, int64_t *n_records);
 /* Extension (the reference requires a coordinate-sorted, indexed BAM): put the records the context holds (every batch
  * pushed so far) into coordinate order on the device.
  * *was_sorted = 1: they already were non-decreasing in (tid as uint32, so tid -1 is last; pos).  Nothing moves: a file
