@@ -3,7 +3,7 @@
 // Same process contract as the reference main() (reference src/BreakID.cc:6-192): flags
 // -i -o -n -q -t -fast -all -h -? (single-dash long options, src/BreakID.cc:15-26), outputs
 // <o>_fusion.txt, <o>_fusion_all.txt (with -all), <o>_params.txt, <o>_performance.txt, error
-// messages + exit(1) as the reference prints them.  Differences, all additive and default-neutral:
+// messages + exit(1) as the reference prints them (exit(-1), status 255, on its fatal "error cigar" path).  Differences, all additive and default-neutral:
 //   * the option table is terminated, so unknown flags report an error instead of segfaulting, and
 //     -t takes its argument (the reference declares has_arg=0 and then reads optarg);
 //   * -s <k>   sd multiplier of the distance formula (the literal 3 at src/BreakID.cc:103);
@@ -381,9 +381,9 @@ int main(int argc, char *argv[])
     std::vector<int64_t> ncall(W);
     double t_run0 = now_s();
     std::cout << "Scanning discordant read pairs ...\n";
-    if (bkid_dist_run_threads(ctxs.data(), comms.data(), W, fast ? 1 : 0, mean.data(), sd.data(), dist.data(), ncall.data())) {
+    if (int rc = bkid_dist_run_threads(ctxs.data(), comms.data(), W, fast ? 1 : 0, mean.data(), sd.data(), dist.data(), ncall.data())) {
       for (int r = 0; r < W; ++r) if (*bkid_last_error(ctxs[r])) std::cerr << "Error: rank " << r << ": " << bkid_last_error(ctxs[r]) << std::endl;
-      exit(1);
+      exit(rc == BKID_ERR_CIGAR ? -1 : 1);
     }
     std::cout << "Scanning discordant read pairs done.\n";
     double t_run = now_s() - t_run0;
@@ -489,7 +489,10 @@ int main(int argc, char *argv[])
         if (bkid_set_nib(ctx, t, nb.payload(), nb.size())) die("set_nib");
     }
     double t1 = now_s();
-    if (bkid_refine(ctx, dist, &n_called)) die("refine");
+    if (int rc = bkid_refine(ctx, dist, &n_called)) {
+      std::cerr << "Error: refine: " << bkid_last_error(ctx) << std::endl;
+      exit(rc == BKID_ERR_CIGAR ? -1 : 1);                                                           // the reference's exit(-1), src/BreakID.cc:954-968
+    }
     t_bp = now_s() - t1;
     cl.resize((size_t)std::max<int64_t>(n_called, 1));
     int64_t n = 0;

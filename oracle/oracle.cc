@@ -95,6 +95,11 @@ static int g_sd_mult = 3;
 void orc_set_sd_mult(int m) { g_sd_mult = m; }
 double orc_dist(double mean, double sd, int times) { return times * sqrt(times) * (mean + g_sd_mult * sd); }
 
+/* the breakpoint vote window (src/BreakID.cc:444-445, literal 2) and the complementary-cigar tolerance (:891, literal 10)
+ * of every refinement entry point; the device reads them from bkid_params.bp_pos_error / mismatch_num */
+static int g_bp_err = 2, g_mismatch = 10;
+void orc_set_refine_consts(int bp_err, int mismatch) { g_bp_err = bp_err; g_mismatch = mismatch; }
+
 /* ------------------------------------------------------------------------------------------
  * a2/a3. discordant-pair scan -- src/BreakID.cc:1362-1515, src/util_bam.cc:7-47,57-68.
  * names[t] = header target name of tid t.  Output: pairs bucket by bucket in std::map<string>
@@ -983,7 +988,7 @@ long orc_find_sa_reads(long n, const uint16_t *flag, const uint8_t *mapq, const 
 {
   Recs R; fill_recs(R, n, flag, mapq, tid, pos, endpos, nh, n_sa, sa_rec, cig_off, cig_ops, sa_off, sa_txt, oc_off, oc_txt);
   std::map<std::pair<uint64_t, uint64_t>, std::vector<Ev>> m; std::vector<Ev> flat;
-  find_sa_reads(R, q_tid, start, end, m, &flat, 10);
+  find_sa_reads(R, q_tid, start, end, m, &flat, g_mismatch);
   orc_evidence *o = (orc_evidence *)calloc(flat.size() ? flat.size() : 1, sizeof(orc_evidence));
   std::vector<std::string> others;
   for (size_t k = 0; k < flat.size(); ++k) ev_to_pod(flat[k], o[k], others);
@@ -1000,10 +1005,10 @@ int orc_find_bp(long n, const uint16_t *flag, const uint8_t *mapq, const int32_t
   Recs R; fill_recs(R, n, flag, mapq, tid, pos, endpos, nh, n_sa, sa_rec, cig_off, cig_ops, sa_off, sa_txt, oc_off, oc_txt);
   std::map<std::pair<uint64_t, uint64_t>, std::vector<Ev>> m1, m2;
   *p1_bp = -1; *p2_bp = -1;
-  find_sa_reads(R, tid1, s1, e1, m1, nullptr, 10);
-  if (!m1.empty()) find_sa_reads(R, tid2, s2, e2, m2, nullptr, 10);
+  find_sa_reads(R, tid1, s1, e1, m1, nullptr, g_mismatch);
+  if (!m1.empty()) find_sa_reads(R, tid2, s2, e2, m2, nullptr, g_mismatch);
   if (m1.empty() || m2.empty()) return 0;
-  return find_bp_pair(m1, m2, chr1, 2, p1_bp, p2_bp);
+  return find_bp_pair(m1, m2, chr1, g_bp_err, p1_bp, p2_bp);
 }
 
 double orc_single_base_depth(long n, const uint16_t *flag, const uint8_t *mapq, const int32_t *tid, const int32_t *pos,
@@ -1094,12 +1099,12 @@ long orc_run(long n, const uint16_t *flag, const uint8_t *mapq, const int32_t *t
         uint32_t r1s = (uint32_t)(c.p1_mean_pos - w), r1e = (uint32_t)(c.p1_mean_pos + w);
         uint32_t r2s = (uint32_t)(c.p2_mean_pos - w), r2e = (uint32_t)(c.p2_mean_pos + w);
         std::map<std::pair<uint64_t, uint64_t>, std::vector<Ev>> m1, m2;
-        find_sa_reads(R, c.p1_tid, r1s, r1e, m1, nullptr, 10);
-        if (!m1.empty()) find_sa_reads(R, c.p2_tid, r2s, r2e, m2, nullptr, 10);
+        find_sa_reads(R, c.p1_tid, r1s, r1e, m1, nullptr, g_mismatch);
+        if (!m1.empty()) find_sa_reads(R, c.p2_tid, r2s, r2e, m2, nullptr, g_mismatch);
         if (m1.empty() || m2.empty()) continue;
         int32_t b1, b2;
         std::string p1name = c.p1_tid >= 0 ? names[c.p1_tid] : "*";
-        int votes = find_bp_pair(m1, m2, p1name, 2, &b1, &b2);
+        int votes = find_bp_pair(m1, m2, p1name, g_bp_err, &b1, &b2);
         if (votes < 2) continue;                                                          /* :446 */
         c.p1_exact_pos = (uint32_t)b1; c.p2_exact_pos = b2; c.n_split_read = votes;
         c.p1_bp_depth = single_base_depth(R, c.p1_tid, (uint64_t)c.p1_exact_pos);
@@ -1308,7 +1313,7 @@ void orc_shard_sa_rows(long n, const uint16_t *flag, const uint8_t *mapq, const 
     sa_c.set_text(f[3]);
     rec_c.set_bam(cig_ops + cig_off[k], (int)(cig_off[k + 1] - cig_off[k]));
     if (!oc.empty()) c1.set_text(oc); else c1 = rec_c;
-    if (!complementary(c1, f[3], 10)) continue;
+    if (!complementary(c1, f[3], g_mismatch)) continue;
     r.ok = 1; r.secondary = (flag[i] & F_SECONDARY) ? 1 : 0;
     uint32_t sa_start = (uint32_t)atoi(f[1].c_str()), sa_end = sa_c.aln_end(sa_start);
     uint32_t a_start = (uint32_t)((long)pos[i] + 1);
@@ -1399,7 +1404,8 @@ long orc_shard_vote(long n_rows, const orc_sarow *rows, long ncl, orc_cluster *c
       size_t q = kv.first.find(',');
       uint32_t k1 = (uint32_t)strtoull(kv.first.substr(0, q).c_str(), nullptr, 10), k2 = (uint32_t)strtoull(kv.first.substr(q + 1).c_str(), nullptr, 10);
       for (auto &u : upd)
-        if (((uint32_t)u.first <= k1 + 2 && (uint32_t)u.first >= k1 - 2) && ((uint32_t)u.second <= k2 + 2 && (uint32_t)u.second >= k2 - 2)) kv.second++;
+        if (((uint32_t)u.first <= k1 + g_bp_err && (uint32_t)u.first >= k1 - g_bp_err) &&
+            ((uint32_t)u.second <= k2 + g_bp_err && (uint32_t)u.second >= k2 - g_bp_err)) kv.second++;
       if (best < kv.second) { best = kv.second; bx = (int32_t)k1; by = (int32_t)k2; }
     }
     if (best >= 2) { valid[c] = 1; cl[c].p1_exact_pos = (uint32_t)bx; cl[c].p2_exact_pos = by; cl[c].n_split_read = best; }

@@ -49,6 +49,7 @@ def olib():
             build(ref=False)
         o = C.CDLL(LIB_ORACLE)
         o.orc_insert_stats.argtypes = [L, u16p, i32p, C.POINTER(D), C.POINTER(D)] + [C.POINTER(C.c_int64)] * 3
+        o.orc_set_refine_consts.argtypes = [I, I]
         o.orc_dist.restype = D
         o.orc_dist.argtypes = [D, D, I]
         o.orc_scan.restype = L
@@ -231,15 +232,40 @@ def sort_perm(key, model=False):
     return perm
 
 
-def find_sa_reads(hb, tid, start, end):
+_refine = [2, 10]                             # the values in force in liboracle (bp_err, mismatch)
+
+
+class refine_consts:
+    """inside the block, every refinement entry point of the oracle (run, find_sa_reads, find_bp and the shard pieces of
+    OracleEngine) votes with a window of +-bp_err and accepts complementary cigars within `mismatch` bases: the literals
+    2 and 10 of src/BreakID.cc:444-445 and :891, bkid_params.bp_pos_error and mismatch_num on the device.  None keeps
+    the value in force; the values in force before the block come back when it ends"""
+
+    def __init__(self, bp_err=None, mismatch=None):
+        self.bp_err, self.mismatch = bp_err, mismatch
+
+    def __enter__(self):
+        self.saved = tuple(_refine)
+        _refine[:] = [self.saved[0] if self.bp_err is None else int(self.bp_err),
+                      self.saved[1] if self.mismatch is None else int(self.mismatch)]
+        olib().orc_set_refine_consts(*_refine)
+
+    def __exit__(self, *a):
+        _refine[:] = self.saved
+        olib().orc_set_refine_consts(*_refine)
+
+
+def find_sa_reads(hb, tid, start, end, mismatch=None):
     out = C.c_void_p()
-    n = olib().orc_find_sa_reads(*_recargs(hb), tid, start, end, C.byref(out))
+    with refine_consts(mismatch=mismatch):
+        n = olib().orc_find_sa_reads(*_recargs(hb), tid, start, end, C.byref(out))
     return _take(out, n, EVIDENCE_DTYPE, olib().orc_free)
 
 
-def find_bp(hb, tid1, s1, e1, tid2, s2, e2):
+def find_bp(hb, tid1, s1, e1, tid2, s2, e2, bp_err=None, mismatch=None):
     a, b = C.c_int32(), C.c_int32()
-    v = olib().orc_find_bp(*_recargs(hb), tid1, hb.target_names[tid1].encode(), s1, e1, tid2, s2, e2, C.byref(a), C.byref(b))
+    with refine_consts(bp_err, mismatch):
+        v = olib().orc_find_bp(*_recargs(hb), tid1, hb.target_names[tid1].encode(), s1, e1, tid2, s2, e2, C.byref(a), C.byref(b))
     return v, a.value, b.value
 
 
@@ -254,12 +280,14 @@ def neighbor_41(packed, nbases, bp):
     return buf.value
 
 
-def run(hb, nibs=None, qual=20, times=2, mode=0, sd_mult=3):
+def run(hb, nibs=None, qual=20, times=2, mode=0, sd_mult=3, bp_err=None, mismatch=None):
     """whole hot path; nibs = list of (packed uint8 array, n_bases) per tid or None.  sd_mult replaces the literal 3 of
-    src/BreakID.cc:103 (the -s extension)"""
+    src/BreakID.cc:103 (the -s extension), bp_err and mismatch the literals 2 and 10 of the refinement (refine_consts;
+    None: the values in force)"""
     olib().orc_set_sd_mult(int(sd_mult))
     try:
-        return _run(hb, nibs, qual, times, mode)
+        with refine_consts(bp_err, mismatch):
+            return _run(hb, nibs, qual, times, mode)
     finally:
         olib().orc_set_sd_mult(3)
 
