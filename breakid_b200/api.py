@@ -184,7 +184,8 @@ class HostBatch:
 
     # -- constructors ----------------------------------------------------------------------
     @staticmethod
-    def from_synth(d) -> "HostBatch":
+    def from_synth(d, target_names=None) -> "HostBatch":
+        """target_names: the header name of every tid (default synth.chrom_name)"""
         from . import synth
         cols = {k: d.cols[k].cpu().numpy() for k in ("mapq", "tid", "pos", "mtid", "mpos", "isize", "endpos")}
         cols["flag"] = d.cols["flag"].cpu().numpy().view(np.uint16)
@@ -192,7 +193,7 @@ class HostBatch:
         side = {"sa_rec": d.sa_rec.cpu().numpy(), "cig_off": d.cig_off.cpu().numpy(),
                 "cig_ops": d.cig_ops.cpu().numpy(), "sa_off": d.sa_off.cpu().numpy(),
                 "sa_txt": d.sa_txt.cpu().numpy()}
-        names = [synth.chrom_name(t) for t in range(len(d.cfg.chrom_lens))]
+        names = [synth.chrom_name(t) for t in range(len(d.cfg.chrom_lens))] if target_names is None else list(target_names)
         return HostBatch(cols, nh, side, d.cfg.chrom_lens, names)
 
     @staticmethod

@@ -39,12 +39,22 @@ def reg2bin(beg: np.ndarray, end: np.ndarray) -> np.ndarray:
     return out
 
 
+def _names(d: synth.SynthData, target_names) -> List[str]:
+    n = len(d.cfg.chrom_lens)
+    names = [synth.chrom_name(t) for t in range(n)] if target_names is None else [str(x) for x in target_names]
+    assert len(names) == n, (len(names), n)
+    return names
+
+
 def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: int = 1,
-              chunk: int = 200_000, sa_seq=None, sort_order: str = "coordinate") -> None:
+              chunk: int = 200_000, sa_seq=None, sort_order: str = "coordinate", target_names=None) -> None:
     """``sort_order`` = the @HD SO: value; the records are written in the batch's order whatever it says.
     ``sa_seq`` = optional seq table (seq_off / seq4 / seq_len, see synth.split_read_sequences): real read bases for
-    the SA-tagged records (all other records carry a constant sequence)."""
+    the SA-tagged records (all other records carry a constant sequence).  ``target_names`` = the @SQ name of every
+    tid (default synth.chrom_name); the SA texts are written as the batch holds them, so whoever builds the batch
+    names their chromosomes."""
     cfg = d.cfg
+    names = _names(d, target_names)
     L = cfg.read_len
     c = {k: v.cpu().numpy() for k, v in d.cols.items()}
     n = c["flag"].shape[0]
@@ -62,10 +72,10 @@ def write_bam(path: str, d: synth.SynthData, random_qual: bool = True, level: in
 
     # header
     text = "@HD\tVN:1.4\tSO:%s\n" % sort_order + "".join(
-        "@SQ\tSN:%s\tLN:%d\n" % (synth.chrom_name(t), l) for t, l in enumerate(cfg.chrom_lens))
+        "@SQ\tSN:%s\tLN:%d\n" % (names[t], l) for t, l in enumerate(cfg.chrom_lens))
     hdr = b"BAM\x01" + struct.pack("<i", len(text)) + text.encode() + struct.pack("<i", len(cfg.chrom_lens))
     for t, l in enumerate(cfg.chrom_lens):
-        nm = synth.chrom_name(t).encode() + b"\x00"
+        nm = names[t].encode() + b"\x00"
         hdr += struct.pack("<i", len(nm)) + nm + struct.pack("<i", l)
 
     out = open(path, "wb")
@@ -157,7 +167,7 @@ _NT16 = np.frombuffer(b"=ACMGRSVTWYHKDBN", dtype=np.uint8)
 
 
 def write_sam(path: str, d: synth.SynthData, random_qual: bool = True, chunk: int = 200_000, sa_seq=None,
-              sort_order: str = "coordinate") -> None:
+              sort_order: str = "coordinate", target_names=None) -> None:
     """The records ``write_bam`` writes (same arguments, same names, cigars, SA tags, bases and qualities) as SAM text:
     RNEXT is "=" when the mate is on the record's own target, SEQ spells the 4-bit codes, QUAL is Phred + 33."""
     cfg = d.cfg
@@ -169,7 +179,7 @@ def write_sam(path: str, d: synth.SynthData, random_qual: bool = True, chunk: in
     sa_off = d.sa_off.cpu().numpy(); sa_txt = d.sa_txt.cpu().numpy()
     sa_slot = np.full(n, -1, dtype=np.int64); sa_slot[sa_rec] = np.arange(sa_rec.shape[0])
     rng = np.random.RandomState(cfg.seed + 12345)          # the qualities write_bam draws, in the same order
-    names = [synth.chrom_name(t) for t in range(len(cfg.chrom_lens))]
+    names = _names(d, target_names)
     with open(path, "wb") as out:
         out.write(("@HD\tVN:1.4\tSO:%s\n" % sort_order + "".join("@SQ\tSN:%s\tLN:%d\n" % (names[t], l) for t, l in enumerate(cfg.chrom_lens))).encode())
         plain = "%dM" % L
@@ -204,24 +214,27 @@ def write_sam(path: str, d: synth.SynthData, random_qual: bool = True, chunk: in
 
 
 def write_dataset(dirpath: str, d: synth.SynthData, random_qual: bool = True, nib: bool = True,
-                  genes_per_mb: float = 4.0, sort_order: str = "coordinate", sam: bool = False) -> dict:
+                  genes_per_mb: float = 4.0, sort_order: str = "coordinate", sam: bool = False, target_names=None) -> dict:
     """Lay down everything a BreakID run needs: <dir>/reads.bam, <dir>/nib/{ref_names.txt,
     hg19_<chr>.nib}, <dir>/ref_files/refGene.txt, and with ``sam`` also <dir>/reads.sam (the same records as text).
-    Returns the paths."""
+    ``target_names`` names every tid in the headers, the nib files, ref_names.txt and refGene.txt (default
+    synth.chrom_name).  Returns the paths."""
     import os
     os.makedirs(os.path.join(dirpath, "nib"), exist_ok=True)
     os.makedirs(os.path.join(dirpath, "ref_files"), exist_ok=True)
     cfg = d.cfg
+    names = _names(d, target_names)
     bam = os.path.join(dirpath, "reads.bam")
-    write_bam(bam, d, random_qual=random_qual, sort_order=sort_order)
+    write_bam(bam, d, random_qual=random_qual, sort_order=sort_order, target_names=names)
     paths = {}
     if sam:
         paths["sam"] = os.path.join(dirpath, "reads.sam")
-        write_sam(paths["sam"], d, random_qual=random_qual, sort_order=sort_order)
-    synth.write_ref_names(os.path.join(dirpath, "nib", "ref_names.txt"), len(cfg.chrom_lens))
+        write_sam(paths["sam"], d, random_qual=random_qual, sort_order=sort_order, target_names=names)
+    synth.write_ref_names(os.path.join(dirpath, "nib", "ref_names.txt"), len(cfg.chrom_lens), target_names=names)
     if nib:
         for t, l in enumerate(cfg.chrom_lens):
             pay = synth.random_nib_bytes(l, cfg.seed * 1000 + t)
-            synth.write_nib(os.path.join(dirpath, "nib", "hg19_%s.nib" % synth.chrom_name(t)), pay, l)
-    synth.write_refgene(os.path.join(dirpath, "ref_files", "refGene.txt"), cfg.chrom_lens, genes_per_mb=genes_per_mb)
+            synth.write_nib(os.path.join(dirpath, "nib", "hg19_%s.nib" % names[t]), pay, l)
+    synth.write_refgene(os.path.join(dirpath, "ref_files", "refGene.txt"), cfg.chrom_lens, genes_per_mb=genes_per_mb,
+                        target_names=names)
     return dict({"bam": bam, "nib": os.path.join(dirpath, "nib"), "refgene": os.path.join(dirpath, "ref_files", "refGene.txt")}, **paths)

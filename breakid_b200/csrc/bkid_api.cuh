@@ -586,14 +586,48 @@ void bkid_default_params(bkid_params *p)
   p->qual = 20; p->times = 2; p->fast = 0; p->min_reads = 2; p->bp_pos_error = 2; p->mismatch_num = 10; p->sd_mult = 3; p->validate_align = 0;
 }
 
+// rank of every "A_B" bucket name in std::map<string> order (src/BreakID.cc:1500-1512), rank[a * m + b] with m = nt + 1
+// and index 0 = "*".  Equal strings get one rank: two target pairs whose names concatenate alike ("scaf" + "1_2",
+// "scaf_1" + "2") are one bucket of the reference's map.  Ranks are dense.  Throws std::bad_alloc.
+static void bucket_rank_table(const std::vector<std::string> &names, std::vector<int32_t> &rank)
+{
+  const int m = (int)names.size() + 1;
+  std::vector<std::pair<std::string, int>> bn;
+  bn.reserve((size_t)m * m);
+  for (int a = 0; a < m; ++a)
+    for (int b = 0; b < m; ++b) bn.push_back({(a ? names[a - 1] : std::string("*")) + "_" + (b ? names[b - 1] : std::string("*")), a * m + b});
+  std::sort(bn.begin(), bn.end());
+  rank.assign((size_t)m * m, 0);
+  int32_t r = -1;
+  for (size_t k = 0; k < bn.size(); ++k) {
+    if (k == 0 || bn[k].first != bn[k - 1].first) ++r;
+    rank[bn[k].second] = r;
+  }
+}
+
 bkid_ctx *bkid_create(int device, const bkid_header *hdr, const bkid_params *params)
 {
+  if (!hdr || hdr->n_targets < 0) { g_create_err = "bad header"; return nullptr; }
+  if (hdr->n_targets > BKID_MAX_TARGETS) {             // (n_targets + 1)^2 bucket ranks are indexed as int32
+    g_create_err = "header has " + std::to_string(hdr->n_targets) + " targets; at most " + std::to_string(BKID_MAX_TARGETS) +
+                   " are supported (the bucket-name rank table holds (n_targets + 1)^2 entries)";
+    return nullptr;
+  }
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0) { g_create_err = std::string("no usable CUDA device (there is no CPU fallback): ") + cudaGetErrorString(e); return nullptr; }
   if (device < 0 || device >= ndev) { g_create_err = "device index out of range"; return nullptr; }
-  if (!hdr || hdr->n_targets < 0) { g_create_err = "bad header"; return nullptr; }
   if (cudaSetDevice(device) != cudaSuccess) { g_create_err = "cudaSetDevice failed"; return nullptr; }
+  const int nt = hdr->n_targets;
+  std::vector<std::string> names;
+  std::vector<int32_t> rank;
+  try {
+    for (int i = 0; i < nt; ++i) names.emplace_back(hdr->target_name[i]);
+    bucket_rank_table(names, rank);
+  } catch (const std::bad_alloc &) {
+    g_create_err = "out of host memory building the bucket-name rank table of " + std::to_string(nt) + " targets";
+    return nullptr;
+  }
   bkid_ctx *c = new bkid_ctx();
   c->device = device;
   cudaDeviceGetAttribute(&c->n_sm, cudaDevAttrMultiProcessorCount, device);
@@ -605,18 +639,11 @@ bkid_ctx *bkid_create(int device, const bkid_header *hdr, const bkid_params *par
   for (auto &ev : c->ev_run) cudaEventCreate(&ev);
   for (auto &ev : c->ev_side) cudaEventCreate(&ev);
   for (auto &ev : c->ev_w) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-  c->nt = hdr->n_targets;
-  for (int i = 0; i < c->nt; ++i) { c->target_len.push_back(hdr->target_len[i]); c->names.emplace_back(hdr->target_name[i]); }
-  int nt = c->nt, m = nt + 1;
+  c->nt = nt;
+  c->names = std::move(names);
+  for (int i = 0; i < nt; ++i) c->target_len.push_back(hdr->target_len[i]);
   std::vector<uint32_t> cum(nt + 1, 0);
   for (int i = 0; i < nt; ++i) cum[i + 1] = cum[i] + c->target_len[i];                 // uint32 wrap, src/util_bam.cc:61-64
-  // rank of every "A_B" bucket name in std::map<string> order (src/BreakID.cc:1500-1512); index 0 = "*"
-  std::vector<std::pair<std::string, int>> bn;
-  for (int a = 0; a < m; ++a)
-    for (int b = 0; b < m; ++b) bn.push_back({(a ? c->names[a - 1] : std::string("*")) + "_" + (b ? c->names[b - 1] : std::string("*")), a * m + b});
-  std::sort(bn.begin(), bn.end());
-  std::vector<int32_t> rank((size_t)m * m);
-  for (size_t r = 0; r < bn.size(); ++r) rank[bn[r].second] = (int32_t)r;
   std::vector<uint64_t> canon(nt ? nt : 1);
   for (int i = 0; i < nt; ++i) canon[i] = chr_code((const uint8_t *)c->names[i].data(), (uint32_t)c->names[i].size());
   bool ok = c->d_cum.ensure((size_t)(nt + 1) * 4, 0, c->st) == 0 && c->d_bucket_rank.ensure(rank.size() * 4, 0, c->st) == 0 &&

@@ -546,16 +546,18 @@ def write_nib(path: str, payload: torch.Tensor, length: int):
         f.write(payload.cpu().numpy().tobytes())
 
 
-def write_ref_names(path: str, n_chr: int):
+def write_ref_names(path: str, n_chr: int, target_names=None):
+    """one name per line: target_names[t], or chrom_name(t) without them"""
     with open(path, "w") as f:
         for t in range(n_chr):
-            f.write(chrom_name(t) + "\n")
+            f.write((chrom_name(t) if target_names is None else str(target_names[t])) + "\n")
 
 
-def write_refgene(path: str, chrom_lens: List[int], genes_per_mb: float = 4.0, seed: int = 7):
+def write_refgene(path: str, chrom_lens: List[int], genes_per_mb: float = 4.0, seed: int = 7, target_names=None):
     """Synthetic UCSC refGene.txt (16 tab-separated columns, parsed by the reference at
     src/RefSeqTranscript.cc:19-79).  Every transcript has a CDS (the reference underflows on
-    CDS-less overlaps, src/BreakID.cc:1757) ; a few NR_ rows exercise the skip rule."""
+    CDS-less overlaps, src/BreakID.cc:1757) ; a few NR_ rows exercise the skip rule.  The chromosome column is
+    target_names[tid], or chrom_name(tid) without them."""
     rng = np.random.RandomState(seed)
     rows = []
     gid = 0
@@ -574,7 +576,7 @@ def write_refgene(path: str, chrom_lens: List[int], genes_per_mb: float = 4.0, s
             strand = "+" if rng.rand() < 0.5 else "-"
             name = ("NR_%06d" % gid) if gid % 17 == 0 else ("NM_%06d" % gid)
             rows.append("\t".join([
-                "0", name, chrom_name(tid), strand, str(tx_s), str(tx_e), str(cds_s), str(cds_e), str(ne),
+                "0", name, chrom_name(tid) if target_names is None else str(target_names[tid]), strand, str(tx_s), str(tx_e), str(cds_s), str(cds_e), str(ne),
                 ",".join(map(str, es)) + ",", ",".join(map(str, ee)) + ",", "0", "GENE%d" % gid,
                 "cmpl", "cmpl", ",".join(["0"] * ne) + ","]))
     with open(path, "w") as f:

@@ -178,7 +178,12 @@ int bkid_abi_version(void);
 const char *bkid_last_error(const bkid_ctx *ctx);       /* ctx may be NULL: last create error */
 void bkid_default_params(bkid_params *p);
 
-/* replaces: process start-up in reference main() (src/BreakID.cc:93-112) */
+/* replaces: process start-up in reference main() (src/BreakID.cc:93-112).  The context holds the rank of every
+ * "<name>_<name>" bucket string over the header's targets and "*", (n_targets + 1)^2 entries indexed as int32: a header
+ * with more than BKID_MAX_TARGETS targets, or one whose table does not fit in host memory, makes it return NULL with
+ * the reason in bkid_last_error(NULL).  Equal bucket strings (e.g. "scaf" + "1_2" and "scaf_1" + "2") get one rank,
+ * as they are one bucket of the reference's std::map. */
+#define BKID_MAX_TARGETS 46339
 bkid_ctx *bkid_create(int device, const bkid_header *hdr, const bkid_params *params);
 void bkid_destroy(bkid_ctx *ctx);
 

@@ -161,7 +161,8 @@ long orc_scan(long n, const uint16_t *flag, const uint8_t *mapq, const int32_t *
 
 /* rank of every possible "chrA_chrB" bucket name in std::map<string> order (what the product's
  * host computes once per header and hands to the device).  rank[(a+1)*(n_targets+1)+(b+1)],
- * index 0 = "*". */
+ * index 0 = "*".  Dense: equal strings ("scaf" + "1_2", "scaf_1" + "2") share a rank, as they share
+ * one key of orc_scan's map. */
 void orc_bucket_rank_table(int n_targets, const char *const *names, int32_t *rank)
 {
   int m = n_targets + 1;
@@ -172,7 +173,11 @@ void orc_bucket_rank_table(int n_targets, const char *const *names, int32_t *ran
       v.push_back({sa + "_" + sb, a * m + b});
     }
   std::sort(v.begin(), v.end());
-  for (size_t r = 0; r < v.size(); ++r) rank[v[r].second] = (int32_t)r;
+  int32_t r = -1;
+  for (size_t k = 0; k < v.size(); ++k) {
+    if (k == 0 || v[k].first != v[k - 1].first) ++r;
+    rank[v[k].second] = r;
+  }
 }
 
 /* ------------------------------------------------------------------------------------------

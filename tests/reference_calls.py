@@ -28,12 +28,12 @@ def fusion_all_rows(prefix):
     return rows
 
 
-def match_oracle(prefix, d, mode=0, qual=None, sd_mult=3, check_w=True):
+def match_oracle(prefix, d, mode=0, qual=None, sd_mult=3, check_w=True, target_names=None):
     """assert the driver's files under `prefix` hold the oracle's calls on SynthData `d` (and its w); returns the oracle's
-    (mean, sd, dist)"""
+    (mean, sd, dist).  target_names: the header names the files were written with (default synth.chrom_name)"""
     from breakid_b200 import api, synth
     from test_golden import _format_calls
-    hb = api.HostBatch.from_synth(d)
+    hb = api.HostBatch.from_synth(d, target_names)
     nibs = [(synth.random_nib_bytes(l, d.cfg.seed * 1000 + t).numpy(), l) for t, l in enumerate(d.cfg.chrom_lens)]
     mean, sd, dist, cl = O.run(hb, nibs, mode=mode, sd_mult=sd_mult, **({"qual": qual} if qual is not None else {}))
     assert fusion_all_rows(prefix) == _format_calls(cl, hb.target_names)
