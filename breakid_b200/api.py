@@ -266,6 +266,10 @@ def host_lib():
             fn.restype = rt
             fn.argtypes = [C.c_void_p]
         L.bkid_host_bgzf_close.argtypes = [C.c_void_p]
+        L.bkid_host_bgzf_walk.restype = C.c_int64
+        L.bkid_host_bgzf_walk.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_char_p, C.c_int]
+        L.bkid_host_bgzf_parse.restype = C.c_void_p
+        L.bkid_host_bgzf_parse.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int), C.c_char_p, C.c_int]
         L.bkid_host_sam_open.restype = C.c_void_p
         L.bkid_host_sam_open.argtypes = [C.c_char_p, C.c_char_p, C.c_int]
         L.bkid_host_sam_parse.restype = C.c_void_p
@@ -290,7 +294,8 @@ EXPORTS = ["bkid_abi_version", "bkid_last_error", "bkid_default_params", "bkid_c
            "bkid_shard_finish", "bkid_fetch_bucket_ranks", "bkid_device_copy",
            "bkid_push_bgzf", "bkid_push_bgzf_range", "bkid_get_decode_stats", "bkid_fetch_column", "bkid_set_exclude", "bkid_device_gather_rows", "bkid_op_banded_align", "bkid_profile_kernels", "bkid_profile_report",
            "bkid_comm_nccl_unique_id", "bkid_comm_nccl_init", "bkid_comm_nccl_init_all", "bkid_comm_local_create", "bkid_comm_destroy", "bkid_dist_run", "bkid_dist_run_threads",
-           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table", "bkid_sort_records", "bkid_push_sam"]
+           "bkid_op_summarize", "bkid_set_params", "bkid_lpt_owner_table", "bkid_sort_records", "bkid_push_sam",
+           "bkid_bgzf_stream_begin", "bkid_push_bgzf_stream", "bkid_bgzf_stream_end"]
 
 CAND_BYTES = 48
 SAROW_BYTES = 88
@@ -321,6 +326,9 @@ def cuda_lib():
         L.bkid_push_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_int64, C.c_uint64, C.POINTER(C.c_int64)]
         L.bkid_push_bgzf_range.argtypes = [vp, vp, C.c_uint64, vp, C.c_int64, C.c_uint64, C.c_int64, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.bkid_get_decode_stats.argtypes = [vp, C.POINTER(DecodeStats)]
+        L.bkid_bgzf_stream_begin.argtypes = [vp, C.c_uint64]
+        L.bkid_push_bgzf_stream.argtypes = [vp, vp, C.c_uint64, vp, C.c_int64, C.POINTER(C.c_int64)]
+        L.bkid_bgzf_stream_end.argtypes = [vp, C.POINTER(C.c_int64)]
         L.bkid_push_sam.argtypes = [vp, vp, C.c_uint64, C.c_int64, C.POINTER(C.c_int64)]
         L.bkid_fetch_column.argtypes = [vp, C.c_char_p, vp, C.c_int64, C.POINTER(C.c_int64)]
         L.bkid_reset.argtypes = [vp]
@@ -472,6 +480,45 @@ class BgzfFile:
             pass
 
 
+BLOCK_DTYPE = np.dtype([("payload_off", np.uint64), ("payload_len", np.uint32), ("usize", np.uint32)])
+
+
+def bgzf_walk(buf) -> "tuple[np.ndarray, int]":
+    """the whole BGZF blocks at the front of ``buf`` (``bkid_host_bgzf_walk``): (block table with payload_off relative to
+    buf, bytes they span).  An incomplete trailing block is not consumed; bytes that are not BGZF raise IOError."""
+    lib = host_lib()
+    b = np.frombuffer(bytes(buf), np.uint8)
+    out = np.zeros(len(b) // 28 + 1, BLOCK_DTYPE)
+    n = C.c_int64()
+    err = C.create_string_buffer(256)
+    used = lib.bkid_host_bgzf_walk(b.ctypes.data_as(C.c_void_p), len(b), out.ctypes.data_as(C.c_void_p), out.shape[0], C.byref(n), err, 256)
+    if used < 0:
+        raise IOError("bkid_host_bgzf_walk: " + err.value.decode())
+    return out[:n.value].copy(), int(used)
+
+
+def bgzf_parse_header(buf, blocks: np.ndarray):
+    """the BAM header from the leading blocks of a stream prefix (``bkid_host_bgzf_parse``): None while the blocks end
+    before the header does, else (target_names, target_len, first_record_uoffset).  Not a BAM raises IOError."""
+    lib = host_lib()
+    b = np.frombuffer(bytes(buf), np.uint8)
+    blocks = np.ascontiguousarray(blocks, BLOCK_DTYPE)
+    need = C.c_int()
+    err = C.create_string_buffer(256)
+    h = lib.bkid_host_bgzf_parse(b.ctypes.data_as(C.c_void_p), blocks.ctypes.data_as(C.c_void_p), blocks.shape[0], C.byref(need), err, 256)
+    if not h:
+        if need.value:
+            return None
+        raise IOError("bkid_host_bgzf_parse: " + err.value.decode())
+    try:
+        hd = C.cast(lib.bkid_host_bgzf_header(h), C.POINTER(Header)).contents
+        names = [hd.target_name[i].decode() for i in range(hd.n_targets)]
+        lens = [int(hd.target_len[i]) for i in range(hd.n_targets)]
+        return names, lens, int(lib.bkid_host_bgzf_first_record(h))
+    finally:
+        lib.bkid_host_bgzf_close(h)
+
+
 class SamFile:
     """Host half of the SAM path: mapped SAM file (or a header in a caller's buffer) + the target table of its @SQ
     lines (``bkid_host_sam_open`` / ``bkid_host_sam_parse``, breakid_b200/host/bam_reader.h).  ``text`` is a view of the
@@ -593,6 +640,31 @@ class Context:
             ptr, ln = (C.cast(keep, C.c_void_p).value, len(text)) if data_ptr is None else (data_ptr, size)
         self._chk(self.lib.bkid_push_sam(self.ctx, C.c_void_p(ptr), ln, first_line, C.byref(n)))
         del keep
+        return int(n.value)
+
+    def bgzf_stream_begin(self, first_record: int):
+        """open a BGZF stream session (``bkid_bgzf_stream_begin``); first_record = size of the BAM header"""
+        self._chk(self.lib.bkid_bgzf_stream_begin(self.ctx, first_record))
+
+    def push_bgzf_stream(self, piece, blocks: Optional[np.ndarray] = None, data_ptr=None) -> int:
+        """decode the next whole BGZF blocks of the stream (``bkid_push_bgzf_stream``); returns the records that completed.
+        ``piece`` is bytes (``blocks`` defaults to its walk) or its size when ``data_ptr`` points at the bytes (e.g. pinned)."""
+        if data_ptr is None:
+            keep = np.frombuffer(bytes(piece), np.uint8)
+            ptr, size = keep.ctypes.data, len(keep)
+            if blocks is None:
+                blocks = bgzf_walk(piece)[0]
+        else:
+            ptr, size = data_ptr, int(piece)
+        blocks = np.ascontiguousarray(blocks, BLOCK_DTYPE)
+        n = C.c_int64()
+        self._chk(self.lib.bkid_push_bgzf_stream(self.ctx, C.c_void_p(ptr), size, blocks.ctypes.data_as(C.c_void_p), blocks.shape[0], C.byref(n)))
+        return int(n.value)
+
+    def bgzf_stream_end(self) -> int:
+        """close the session (``bkid_bgzf_stream_end``); returns the records of the whole session"""
+        n = C.c_int64()
+        self._chk(self.lib.bkid_bgzf_stream_end(self.ctx, C.byref(n)))
         return int(n.value)
 
     def decode_stats(self) -> dict:

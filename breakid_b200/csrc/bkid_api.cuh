@@ -41,6 +41,9 @@ struct Scratch {          // reusable device scratch for sorts / scans over `cap
 
 struct bkid_decoder;
 static void decoder_free(bkid_ctx *c);
+static bool stream_open(const bkid_ctx *c);     // a BGZF stream session (bkid_bgzf_stream_begin) is open: no other push, sort or stage call
+static void stream_close(bkid_ctx *c);
+#define NO_STREAM(c) do { if (stream_open(c)) return fail((c), BKID_ERR_ARG, "a BGZF stream session is open on this context (bkid_bgzf_stream_end or bkid_reset first)"); } while (0)
 
 struct bkid_ctx {
   bkid_decoder *dec = nullptr;              // streaming BGZF/BAM decode state (bkid_bamdec.cuh)
@@ -797,6 +800,7 @@ static int push_impl(bkid_ctx *c, const bkid_batch *b, cudaMemcpyKind kind)
     return fail(c, BKID_ERR_ARG, "bad batch: a dense column is missing in both its wide and its narrow form");
   cudaSetDevice(c->device);
   cudaStream_t st = c->st;
+  NO_STREAM(c);
   if ((unsigned long long)(c->n + b->n) >= 0xffffffffull) return fail(c, BKID_ERR_ARG, "more than 2^32-1 records per context");
   invalidate(c);
   cudaEventRecord(c->ev[0], st);
@@ -910,6 +914,7 @@ int bkid_push_batch(bkid_ctx *c, const bkid_batch *b) { return push_impl(c, b, c
 int bkid_push_batch_device(bkid_ctx *c, const bkid_batch *b)
 {
   if (!c || !b) return BKID_ERR_ARG;
+  NO_STREAM(c);
   if (c->n == 0 && !c->borrowed && c->flag.p == nullptr) {
     // adopt the caller's device columns without copying (already-resident input), in whichever form they are
     cudaSetDevice(c->device);
@@ -938,6 +943,7 @@ int bkid_reset(bkid_ctx *c)
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->st);
   invalidate(c);
+  stream_close(c);
   c->n = c->n_x = c->n_sa = c->n_cig = c->sa_bytes = c->oc_bytes = 0;
   c->seq_bytes = 0; c->have_seq = false;
   c->borrowed = false;
@@ -974,6 +980,7 @@ static ISizeCol isize_col(const bkid_ctx *c) { return ISizeCol{c->p_isize, c->p_
 static int classify_impl(bkid_ctx *c)
 {
   if (c->classified) return 0;
+  NO_STREAM(c);
   cudaStream_t st = c->st;
   long long n = c->n;
   int ntiles = div_up(std::max<long long>(n, 1), K1_TILE);
@@ -1742,6 +1749,7 @@ int bkid_shard_join(bkid_ctx *c, const bkid_cand *dev_cand, int64_t n, double w,
 int bkid_shard_set_pairs(bkid_ctx *c, const bkid_pair *dev_pairs, int64_t n)
 {
   if (!c) return BKID_ERR_ARG;
+  NO_STREAM(c);
   cudaSetDevice(c->device); c->err.clear();
   TRY(c, set_pairs(c, dev_pairs, n, false));
   c->tm.n_pairs = c->np0;
@@ -2089,6 +2097,7 @@ int bkid_op_cluster(bkid_ctx *c, int mode, int64_t n, const uint32_t *p1, const 
 int bkid_op_summarize(bkid_ctx *c, int64_t n, const bkid_pair *pairs, double dist, int64_t *n_clusters)
 {
   if (!c || n < 0 || (n > 0 && !pairs)) return BKID_ERR_ARG;
+  NO_STREAM(c);
   cudaSetDevice(c->device);
   c->err.clear();
   cudaStream_t st = c->st;

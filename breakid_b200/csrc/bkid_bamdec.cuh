@@ -344,9 +344,28 @@ __global__ void bam_extract_side(const uint8_t *__restrict__ u, const uint32_t *
 
 }  // namespace bamdec
 
+// where the decode of one BGZF stream stands between two chunks; a stream session keeps it between calls
+struct BgzfCursor {
+  uint32_t carry = 0;                   // bytes of the partial record at the end of the last chunk (held in bkid_decoder::carry)
+  uint64_t skip = 0;                    // BAM header bytes still to skip before the first record
+  uint64_t u0 = 0;                      // stream offset of the next uncompressed byte
+  int64_t blk0 = 0;                     // stream index of blocks[0] of the current call (error messages)
+  bool seek = false;                    // block range that starts mid-stream: find the first record by seeding
+  bool range_done = false;              // block range: the walk reached the record that starts the next range
+};
+
+// bkid_bgzf_stream_begin .. bkid_bgzf_stream_end: the cursor and what the context held at begin (restored on any error)
+struct BgzfStream {
+  bool open = false;
+  BgzfCursor cur;
+  long long n = 0, n_x = 0, n_sa = 0, n_cig = 0, sa_b = 0, oc_b = 0, seq_b = 0;
+  bool have_seq = false;
+};
+
 struct bkid_decoder {                 // per-context streaming state, allocated on first use
   DBuf comp[2], unc, carry, tasks, seed, cnt, land, base, rec_off, meta[8], metao[6], state;
-  uint8_t *h_stage[2] = {nullptr, nullptr}; size_t h_cap = 0;
+  uint8_t *h_stage[2] = {nullptr, nullptr}; size_t h_cap = 0; int h_slots = 0;   // pinned staging of pageable input
+  BgzfStream stream;
   bamdec::Task *h_tasks = nullptr; size_t h_tasks_cap = 0;
   cudaStream_t st_copy = nullptr;
   cudaEvent_t ev_h2d[2], ev_free[2], ev_t[8];
@@ -388,24 +407,36 @@ static void decoder_free(bkid_ctx *c)
   c->dec = nullptr;
 }
 
-// Decode the records that START in the uncompressed extent of blocks [b_begin, b_end).  b_begin == 0: the chain starts at
-// first_record_uoffset; otherwise the first record is found by seeding (and reported in *first_uoff so that the caller
-// can verify it against where the previous range landed).  b_end < n_blocks: up to `overlap` further blocks are read
-// so that the record straddling the range end completes; *land_uoff = start of the first record of the NEXT range.
-static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, const bkid_bgzf_block *blocks, int64_t n_blocks, uint64_t first_record_uoffset, int64_t b_begin, int64_t b_end,
-                          int64_t *n_records, uint64_t *first_uoff, uint64_t *land_uoff)
+static bool stream_open(const bkid_ctx *c) { return c->dec && c->dec->stream.open; }
+static void stream_close(bkid_ctx *c) { if (c->dec) c->dec->stream.open = false; }
+
+// pinned staging for pageable input: `slots` buffers of at least `bytes`, kept for later calls; growth is geometric so
+// that a stream of pieces of similar size allocates once
+static int ensure_staging(bkid_ctx *c, size_t bytes, int slots)
+{
+  bkid_decoder *d = c->dec;
+  if (d->h_cap >= bytes && d->h_slots >= slots) return 0;
+  const size_t cap = d->h_cap >= bytes ? d->h_cap : std::max(bytes, d->h_cap + d->h_cap / 2);
+  for (int i = 0; i < 2; ++i) { if (d->h_stage[i]) cudaFreeHost(d->h_stage[i]); d->h_stage[i] = nullptr; }
+  d->h_cap = 0; d->h_slots = 0;
+  for (int i = 0; i < slots; ++i) CU(c, cudaMallocHost((void **)&d->h_stage[i], cap));
+  d->h_cap = cap; d->h_slots = slots;
+  return 0;
+}
+
+// Decode the records that START in the uncompressed extent of blocks [b_begin, b_end) of `file` and append them to the
+// context: the whole-file, block-range and stream calls all run this.  `cur` says where the stream stands before the
+// call (carried partial record, header bytes to skip, stream offset) and where it stands after.  b_begin > 0 (range
+// form): the first record is found by seeding (and reported in *first_uoff so that the caller can verify it against
+// where the previous range landed).  b_end < n_blocks: up to `overlap` further blocks are read so that the record
+// straddling the range end completes; *land_uoff = start of the first record of the NEXT range.  `extrapolate`: the
+// table is the whole stream, so the first chunk sizes the columns for all of it.
+static int decode_blocks(bkid_ctx *c, const uint8_t *file, uint64_t file_size, const bkid_bgzf_block *blocks, int64_t n_blocks, int64_t b_begin, int64_t b_end,
+                         BgzfCursor &cur, bool extrapolate, uint64_t *first_uoff, uint64_t *land_uoff)
 {
   using namespace bamdec;
-  if (!c || !file || !blocks || n_blocks < 0 || b_begin < 0 || b_end < b_begin || b_end > n_blocks) return c ? fail(c, BKID_ERR_ARG, "bad bgzf arguments") : BKID_ERR_ARG;
-  cudaSetDevice(c->device);
-  c->err.clear();
-  if (c->borrowed) return fail(c, BKID_ERR_ARG, "context holds borrowed device columns; bkid_reset first");
-  TRY(c, decoder_init(c));
   bkid_decoder *d = c->dec;
   cudaStream_t st = c->st;
-  invalidate(c);
-  TRY(c, settle_forms(c, 1, 1, 0));                           // the decoder writes the wide insert-size / end columns
-  memset(&d->stats, 0, sizeof d->stats);
   d->skip_crc = getenv("BKID_BGZF_NO_CRC") != nullptr;
   size_t COMP_CAP = (size_t)1536 << 20, UNC_CAP = (size_t)3072 << 20, CARRY_CAP = (size_t)64 << 20;   // unc offsets are 32-bit: UNC_CAP + CARRY_CAP < 4 GiB
   if (const char *e = getenv("BKID_BGZF_CHUNK_KB")) {          // tests: small chunks exercise the streaming / carry logic on small files
@@ -425,7 +456,7 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
   size_t max_span = 0, max_unc = 0;
   const int64_t OVERLAP = 64;                               // blocks read past the range end for the straddling record (4 MiB)
   const int64_t b_last = b_end < n_blocks ? std::min<int64_t>(n_blocks, b_end + OVERLAP) : n_blocks;
-  uint64_t u_begin = 0, u_end = 0;                          // uncompressed offsets of the range in the whole stream
+  uint64_t u_begin = cur.u0, u_end = cur.u0;                // uncompressed offsets of the range in the whole stream
   for (int64_t b = 0; b < b_end; ++b) { if (b < b_begin) u_begin += blocks[b].usize; u_end += blocks[b].usize; }
   const bool open_end = b_end >= n_blocks;
   for (int64_t b0 = b_begin; b0 < b_last;) {
@@ -451,14 +482,10 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
   // buffers are sized by what this file needs (small files: small allocations); the carry buffer grows on demand
   size_t carry_cap = std::min<size_t>(CARRY_CAP, (size_t)4 << 20);
   TRY(c, d->unc.ensure(max_unc + CARRY_CAP + 256, 0, st));
-  TRY(c, d->carry.ensure(carry_cap + 256, 0, st));
+  TRY(c, d->carry.ensure(carry_cap + 256, cur.carry, st));
   TRY(c, d->state.ensure(256, 0, st));
   for (int i = 0; i < (chunks.size() > 1 ? 2 : 1); ++i) TRY(c, d->comp[i].ensure(max_span + 256, 0, st));
-  if (!pinned && d->h_cap < max_span + 256) {
-    for (int i = 0; i < 2; ++i) { if (d->h_stage[i]) cudaFreeHost(d->h_stage[i]); d->h_stage[i] = nullptr; }
-    for (int i = 0; i < (chunks.size() > 1 ? 2 : 1); ++i) CU(c, cudaMallocHost((void **)&d->h_stage[i], max_span + 256));
-    d->h_cap = chunks.size() > 1 ? max_span + 256 : 0;          // a single-slot allocation is not reused for multi-chunk files
-  }
+  if (!pinned && !chunks.empty()) TRY(c, ensure_staging(c, max_span + 256, chunks.size() > 1 ? 2 : 1));
   size_t max_tasks = 0;
   for (auto &ch : chunks) max_tasks = std::max<size_t>(max_tasks, (size_t)(ch.second - ch.first));
   if (d->h_tasks_cap < 2 * max_tasks + 2) {
@@ -492,14 +519,13 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
   for (int i = 0; i < 2; ++i) { CU(c, cudaEventRecord(d->ev_free[i], st)); CU(c, cudaEventRecord(d->ev_h2d[i], d->st_copy)); }
   cudaEventRecord(d->ev_t[0], st);
   if (!chunks.empty()) TRY(c, stage_chunk(0));
-  uint32_t carry = 0;
-  uint64_t skip = b_begin == 0 ? first_record_uoffset : 0;      // bytes of the uncompressed stream before the first record (BAM header)
-  bool seek = b_begin > 0;                         // the first record of a mid-stream range is found by seeding
-  bool range_done = false;
-  uint64_t chunk_u0 = u_begin;                     // stream offset of the first NEW byte of the current chunk
-  if (first_uoff) *first_uoff = first_record_uoffset;
+  uint32_t &carry = cur.carry;
+  uint64_t &skip = cur.skip;
+  bool &seek = cur.seek, &range_done = cur.range_done;
+  uint64_t &chunk_u0 = cur.u0;                     // stream offset of the first NEW byte of the current chunk
+  chunk_u0 = u_begin;
   if (land_uoff) *land_uoff = 0;
-  long long n_first = c->n;
+  const long long n_first = c->n;
   float ms_inf = 0, ms_bound = 0, ms_ext = 0;
   for (size_t k = 0; k < chunks.size() && !range_done; ++k) {
     int slot = (int)(k & 1);
@@ -513,7 +539,7 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
       if (blocks[b].usize) { ht[nt++] = Task{blocks[b].payload_off - span0, uo, blocks[b].payload_len, blocks[b].usize}; task_block.push_back(b); }
       uo += blocks[b].usize;
     }
-    auto block_of = [&](long long t) -> long long { return t >= 0 && t < (long long)task_block.size() ? (long long)task_block[(size_t)t] : (long long)b0 + t; };
+    auto block_of = [&](long long t) -> long long { return cur.blk0 + (t >= 0 && t < (long long)task_block.size() ? (long long)task_block[(size_t)t] : (long long)b0 + t); };
     uint32_t total = uo;
     uint8_t *u = d->unc.as<uint8_t>();
     Task *dt = d->tasks.as<Task>() + (size_t)slot * max_tasks;
@@ -538,6 +564,7 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
       if (skip >= total) { skip -= total; carry = 0; TRY(c, sync_check(c)); continue; }
       start = (uint32_t)skip; skip = 0;
     }
+    if (start >= total) { carry = 0; TRY(c, sync_check(c)); continue; }   // no record bytes: empty blocks only, or the header ends here
     uint32_t nseg = (total + SEG - 1) / SEG;
     // segments before `start` hold header bytes only
     uint32_t seg0 = start / SEG;
@@ -595,7 +622,7 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
     if (nrec) {
       // capacity: after the first chunk extrapolate from records per uncompressed byte
       long long want = c->n + nrec;
-      if (k == 0 && chunks.size() > 1 && total > start) want = std::max<long long>(want, c->n + (long long)((double)nrec / (double)(total - start) * (double)total_u * 1.03) + 1024);
+      if (extrapolate && k == 0 && chunks.size() > 1 && total > start) want = std::max<long long>(want, c->n + (long long)((double)nrec / (double)(total - start) * (double)total_u * 1.03) + 1024);
       want = std::min<long long>(want, 0xfffffffell);
       TRY(c, reserve_impl(c, std::max<long long>(want, c->n + nrec), c->n_x, std::max<long long>(c->n_sa, 1), std::max<long long>(c->n_cig, 1), std::max<long long>(c->sa_bytes, 1), std::max<long long>(c->oc_bytes, 1)));
       TRY(c, d->rec_off.ensure((size_t)nrec * 4 + 64, 0, st));
@@ -655,18 +682,42 @@ static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, 
     cudaEventElapsedTime(&ms, d->ev_t[2], d->ev_t[3]); ms_bound += ms;
     cudaEventElapsedTime(&ms, d->ev_t[3], d->ev_t[4]); ms_ext += ms;
   }
-  if (!open_end && !range_done) return fail(c, BKID_ERR_IO, "the record straddling the end of the block range does not complete within the overlap");
-  if (carry) return fail(c, BKID_ERR_IO, "truncated BAM record at the end of the file");
-  if (open_end && land_uoff) *land_uoff = chunk_u0;
-  if (skip) return fail(c, BKID_ERR_IO, "first_record_uoffset beyond the end of the uncompressed stream");
   cudaEventRecord(d->ev_t[5], st);
   TRY(c, sync_check(c));
   CU(c, cudaStreamSynchronize(d->st_copy));
+  float ms_total = 0;
+  cudaEventElapsedTime(&ms_total, d->ev_t[0], d->ev_t[5]);
+  d->stats.total_ms += ms_total; d->stats.inflate_ms += ms_inf; d->stats.boundaries_ms += ms_bound; d->stats.extract_ms += ms_ext;
+  d->stats.n_records += c->n - n_first;
+  d->stats.n_chunks += (int64_t)chunks.size();
+  cur.blk0 += n_blocks;
+  return 0;
+}
+
+static int push_bgzf_impl(bkid_ctx *c, const uint8_t *file, uint64_t file_size, const bkid_bgzf_block *blocks, int64_t n_blocks, uint64_t first_record_uoffset, int64_t b_begin, int64_t b_end,
+                          int64_t *n_records, uint64_t *first_uoff, uint64_t *land_uoff)
+{
+  if (!c || !file || !blocks || n_blocks < 0 || b_begin < 0 || b_end < b_begin || b_end > n_blocks) return c ? fail(c, BKID_ERR_ARG, "bad bgzf arguments") : BKID_ERR_ARG;
+  cudaSetDevice(c->device);
+  c->err.clear();
+  if (c->borrowed) return fail(c, BKID_ERR_ARG, "context holds borrowed device columns; bkid_reset first");
+  NO_STREAM(c);
+  TRY(c, decoder_init(c));
+  invalidate(c);
+  TRY(c, settle_forms(c, 1, 1, 0));                           // the decoder writes the wide insert-size / end columns
+  memset(&c->dec->stats, 0, sizeof c->dec->stats);
+  BgzfCursor cur;
+  cur.skip = b_begin == 0 ? first_record_uoffset : 0;         // bytes of the uncompressed stream before the first record (BAM header)
+  cur.seek = b_begin > 0;                                     // the first record of a mid-stream range is found by seeding
+  if (first_uoff) *first_uoff = first_record_uoffset;
+  const long long n_first = c->n;
+  TRY(c, decode_blocks(c, file, file_size, blocks, n_blocks, b_begin, b_end, cur, true, first_uoff, land_uoff));
+  const bool open_end = b_end >= n_blocks;
+  if (!open_end && !cur.range_done) return fail(c, BKID_ERR_IO, "the record straddling the end of the block range does not complete within the overlap");
+  if (cur.carry) return fail(c, BKID_ERR_IO, "truncated BAM record at the end of the file");
+  if (open_end && land_uoff) *land_uoff = cur.u0;
+  if (cur.skip) return fail(c, BKID_ERR_IO, "first_record_uoffset beyond the end of the uncompressed stream");
   set_ptrs(c);
-  cudaEventElapsedTime(&d->stats.total_ms, d->ev_t[0], d->ev_t[5]);
-  d->stats.inflate_ms = ms_inf; d->stats.boundaries_ms = ms_bound; d->stats.extract_ms = ms_ext;
-  d->stats.n_records = c->n - n_first;
-  d->stats.n_chunks = (int64_t)chunks.size();
   c->have_seq = true;                    // the decoder always extracts the read bases of the SA records
   if (n_records) *n_records = c->n - n_first;
   return 0;
@@ -681,6 +732,75 @@ int bkid_push_bgzf_range(bkid_ctx *c, const uint8_t *file, uint64_t file_size, c
                          int64_t *n_records, uint64_t *first_record_uoff, uint64_t *next_record_uoff)
 {
   return push_bgzf_impl(c, file, file_size, blocks, n_blocks, first_record_uoffset, first_block, end_block, n_records, first_record_uoff, next_record_uoff);
+}
+
+// ---- BGZF stream (a BAM on a pipe): the whole-file decode, one piece at a time ----------------------------------------
+// Records are only ever appended, so an error restores the counts taken at begin and every column reads as it did then.
+static int stream_abort(bkid_ctx *c, int rc)
+{
+  BgzfStream &s = c->dec->stream;
+  cudaStreamSynchronize(c->st);
+  cudaStreamSynchronize(c->dec->st_copy);
+  c->n = s.n; c->n_x = s.n_x; c->n_sa = s.n_sa; c->n_cig = s.n_cig; c->sa_bytes = s.sa_b; c->oc_bytes = s.oc_b; c->seq_bytes = s.seq_b;
+  c->have_seq = s.have_seq;
+  s.open = false;
+  set_ptrs(c);
+  return rc;
+}
+
+int bkid_bgzf_stream_begin(bkid_ctx *c, uint64_t first_record_uoffset)
+{
+  if (!c) return BKID_ERR_ARG;
+  cudaSetDevice(c->device);
+  c->err.clear();
+  if (c->borrowed) return fail(c, BKID_ERR_ARG, "context holds borrowed device columns; bkid_reset first");
+  NO_STREAM(c);
+  TRY(c, decoder_init(c));
+  invalidate(c);
+  TRY(c, settle_forms(c, 1, 1, 0));                           // the decoder writes the wide insert-size / end columns
+  BgzfStream &s = c->dec->stream;
+  s.cur = BgzfCursor();
+  s.cur.skip = first_record_uoffset;
+  s.n = c->n; s.n_x = c->n_x; s.n_sa = c->n_sa; s.n_cig = c->n_cig; s.sa_b = c->sa_bytes; s.oc_b = c->oc_bytes; s.seq_b = c->seq_bytes;
+  s.have_seq = c->have_seq;
+  memset(&c->dec->stats, 0, sizeof c->dec->stats);
+  s.open = true;
+  return 0;
+}
+
+int bkid_push_bgzf_stream(bkid_ctx *c, const uint8_t *piece, uint64_t piece_size, const bkid_bgzf_block *blocks, int64_t n_blocks, int64_t *n_records)
+{
+  if (!c) return BKID_ERR_ARG;
+  cudaSetDevice(c->device);
+  c->err.clear();
+  if (n_records) *n_records = 0;
+  if (!stream_open(c)) return fail(c, BKID_ERR_ARG, "bkid_push_bgzf_stream without bkid_bgzf_stream_begin");
+  if (n_blocks < 0 || (n_blocks && (!piece || !blocks))) return stream_abort(c, fail(c, BKID_ERR_ARG, "bad bgzf stream arguments"));
+  const long long n0 = c->n;
+  if (int rc = decode_blocks(c, piece, piece_size, blocks, n_blocks, 0, n_blocks, c->dec->stream.cur, false, nullptr, nullptr)) {
+    if (c->err.empty()) c->err = g_last_cuda_err;
+    return stream_abort(c, rc);
+  }
+  set_ptrs(c);
+  if (n_records) *n_records = c->n - n0;
+  return 0;
+}
+
+int bkid_bgzf_stream_end(bkid_ctx *c, int64_t *n_records)
+{
+  if (!c) return BKID_ERR_ARG;
+  cudaSetDevice(c->device);
+  c->err.clear();
+  if (n_records) *n_records = 0;
+  if (!stream_open(c)) return fail(c, BKID_ERR_ARG, "bkid_bgzf_stream_end without bkid_bgzf_stream_begin");
+  BgzfStream &s = c->dec->stream;
+  if (s.cur.carry) return stream_abort(c, fail(c, BKID_ERR_IO, "truncated BAM record at the end of the file"));
+  if (s.cur.skip) return stream_abort(c, fail(c, BKID_ERR_IO, "first_record_uoffset beyond the end of the uncompressed stream"));
+  s.open = false;
+  set_ptrs(c);
+  c->have_seq = true;                    // the decoder always extracts the read bases of the SA records
+  if (n_records) *n_records = c->n - s.n;
+  return 0;
 }
 
 int bkid_get_decode_stats(bkid_ctx *c, bkid_decode_stats *s)

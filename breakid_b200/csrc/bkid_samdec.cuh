@@ -433,11 +433,7 @@ static int push_sam_impl(bkid_ctx *c, const uint8_t *text, uint64_t len, int64_t
   }
   const int slots = chunks.size() > 1 ? 2 : 1;
   for (int k = 0; k < slots; ++k) TRY(c, d->comp[k].ensure(max_chunk + 256, 0, st));
-  if (!pinned && !chunks.empty() && d->h_cap < max_chunk + 256) {   // same staging rule as push_bgzf_impl
-    for (int k = 0; k < 2; ++k) { if (d->h_stage[k]) cudaFreeHost(d->h_stage[k]); d->h_stage[k] = nullptr; }
-    for (int k = 0; k < slots; ++k) CU(c, cudaMallocHost((void **)&d->h_stage[k], max_chunk + 256));
-    d->h_cap = slots > 1 ? max_chunk + 256 : 0;
-  }
+  if (!pinned && !chunks.empty()) TRY(c, ensure_staging(c, max_chunk + 256, slots));
   TRY(c, d->state.ensure(256, 0, st));
   unsigned long long *derr = (unsigned long long *)d->state.as<int>() + 8;
   unsigned long long *tot = (unsigned long long *)(c->counters.as<unsigned>() + CS_TOTAL);
@@ -555,6 +551,7 @@ int bkid_push_sam(bkid_ctx *c, const uint8_t *text, uint64_t len, int64_t first_
   cudaSetDevice(c->device);
   c->err.clear();
   if (c->borrowed) return fail(c, BKID_ERR_ARG, "context holds borrowed device columns; bkid_reset first");
+  NO_STREAM(c);
   // records are only ever appended: a failed call restores the counts and leaves every column as it was
   const long long n = c->n, n_x = c->n_x, n_sa = c->n_sa, n_cig = c->n_cig, sa_b = c->sa_bytes, oc_b = c->oc_bytes, seq_b = c->seq_bytes;
   int rc = push_sam_impl(c, text, len, first_line);

@@ -210,6 +210,7 @@ extern "C" {
 int bkid_sort_records(bkid_ctx *c, int32_t *was_sorted)
 {
   if (!c) return BKID_ERR_ARG;
+  NO_STREAM(c);
   cudaSetDevice(c->device);
   cudaStream_t st = c->st;
   const long long n = c->n, nx = c->n_x, ns = c->n_sa;

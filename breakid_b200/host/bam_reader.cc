@@ -16,6 +16,7 @@
 #include <unistd.h>
 #include <zlib.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cstdio>
 #include <cstring>
@@ -332,6 +333,7 @@ extern "C" void bkid_host_bam_free(bkid_host_bam *h) { delete h; }
 // ---- host half of the device decode path ----------------------------------------------------------------
 struct bkid_host_bgzf {
   const uint8_t *file = nullptr; size_t fsz = 0;
+  bool mapped = false;
   std::vector<bkid_bgzf_block> blocks;
   std::vector<uint32_t> target_len;
   std::vector<std::string> names;
@@ -340,6 +342,113 @@ struct bkid_host_bgzf {
   uint64_t first_record = 0, usize = 0;
   int32_t first_l_qseq = -1;
 };
+
+// the one BGZF block walker (SAM spec 4.1): the whole blocks at the front of buf[0, len) are appended to `out` with
+// payload_off relative to buf; returns the bytes they span (an incomplete trailing block is not consumed), or -1 with
+// `msg` when a block header is not BGZF (magic, FEXTRA, BC subfield, BSIZE)
+static int64_t bgzf_walk(const uint8_t *buf, uint64_t len, std::vector<bkid_bgzf_block> &out, std::string &msg)
+{
+  uint64_t off = 0;
+  while (off + 18 <= len) {
+    const uint8_t *p = buf + off;
+    if (p[0] != 0x1f || p[1] != 0x8b) { msg = "not a BGZF file"; return -1; }
+    if (!(p[3] & 4)) { msg = "corrupt BGZF block (no extra field: plain gzip is not BGZF)"; return -1; }
+    uint16_t xlen = rd16(p + 10);
+    if (off + 12 + xlen > len) break;
+    uint32_t bsize = 0;
+    for (uint32_t x = 0; x + 4 <= xlen;) {        // find the BC subfield (every subfield must lie inside XLEN)
+      const uint8_t *q = p + 12 + x;
+      uint16_t slen = rd16(q + 2);
+      if (x + 4 + (uint32_t)slen > xlen) break;
+      if (q[0] == 'B' && q[1] == 'C' && slen == 2) bsize = (uint32_t)rd16(q + 4) + 1;
+      x += 4 + slen;
+    }
+    if (!bsize || bsize < 12u + xlen + 8u) { msg = "corrupt BGZF block (no BC subfield or BSIZE too small)"; return -1; }
+    if (off + bsize > len) break;
+    bkid_bgzf_block b;
+    b.payload_off = off + 12 + xlen; b.payload_len = bsize - 12 - xlen - 8; b.usize = rd32(p + bsize - 4);
+    out.push_back(b);
+    off += bsize;
+  }
+  return (int64_t)off;
+}
+
+// BAM header (SAM spec 4.2) from the leading blocks: zlib on just enough of them.  1 = parsed, 0 = the blocks end
+// before the header does (need more bytes; `complete` = they are the whole stream: an error instead), -1 = error in msg
+static int bam_header_parse(bkid_host_bgzf *h, const uint8_t *buf, const bkid_bgzf_block *blocks, int64_t n_blocks, bool complete, std::string &msg)
+{
+  std::vector<uint8_t> u;
+  int64_t nb = 0;
+  bool bad = false;
+  auto need = [&](size_t bytes) -> bool {
+    while (u.size() < bytes && nb < n_blocks && !bad) {
+      const bkid_bgzf_block &b = blocks[nb++];
+      size_t o = u.size();
+      u.resize(o + b.usize);
+      if (b.usize) {
+        z_stream zs; memset(&zs, 0, sizeof zs);
+        if (inflateInit2(&zs, -15) != Z_OK) { bad = true; break; }
+        zs.next_in = const_cast<uint8_t *>(buf + b.payload_off); zs.avail_in = b.payload_len;
+        zs.next_out = u.data() + o; zs.avail_out = b.usize;
+        int r = inflate(&zs, Z_FINISH);
+        inflateEnd(&zs);
+        if (r != Z_STREAM_END || zs.total_out != b.usize) bad = true;
+      }
+    }
+    return !bad && u.size() >= bytes;
+  };
+  auto short_of = [&](const char *what) -> int {             // the data ran out (or did not inflate) before `bytes`
+    if (bad || complete) { msg = what; return -1; }
+    return 0;
+  };
+  h->names.clear(); h->target_len.clear(); h->name_ptrs.clear();
+  if (!need(12)) return short_of("not a BAM file");
+  if (memcmp(u.data(), "BAM\1", 4) != 0) { msg = "not a BAM file"; return -1; }
+  size_t o = 4;
+  uint32_t l_text = rd32(u.data() + o); o += 4;
+  if (!need(o + l_text + 4)) return short_of("truncated BAM header");
+  o += l_text;
+  uint32_t n_ref = rd32(u.data() + o); o += 4;
+  for (uint32_t i = 0; i < n_ref; ++i) {
+    if (!need(o + 4)) return short_of("truncated BAM header");
+    uint32_t l_name = rd32(u.data() + o); o += 4;
+    if (!need(o + l_name + 4)) return short_of("truncated BAM header");
+    h->names.emplace_back((const char *)(u.data() + o)); o += l_name;
+    h->target_len.push_back(rd32(u.data() + o)); o += 4;
+  }
+  h->first_record = o;
+  if (need(o + 36)) h->first_l_qseq = (int32_t)rd32(u.data() + o + 20);
+  for (auto &s : h->names) h->name_ptrs.push_back(s.c_str());
+  h->hdr.n_targets = (int32_t)h->names.size();
+  h->hdr.target_len = h->target_len.data();
+  h->hdr.target_name = h->name_ptrs.data();
+  return 1;
+}
+
+extern "C" int64_t bkid_host_bgzf_walk(const uint8_t *buf, uint64_t len, bkid_bgzf_block *out, int64_t cap, int64_t *n_blocks, char *err, int errlen)
+{
+  std::vector<bkid_bgzf_block> v;
+  std::string msg;
+  int64_t used = bgzf_walk(buf, len, v, msg);
+  if (used < 0) { set_err(err, errlen, msg); if (n_blocks) *n_blocks = 0; return -1; }
+  if ((int64_t)v.size() > cap) {                             // a table that does not fit: consume only the blocks it holds
+    v.resize((size_t)std::max<int64_t>(cap, 0));
+    used = v.empty() ? 0 : (int64_t)(v.back().payload_off + v.back().payload_len + 8);
+  }
+  if (!v.empty()) memcpy(out, v.data(), v.size() * sizeof(bkid_bgzf_block));
+  if (n_blocks) *n_blocks = (int64_t)v.size();
+  return used;
+}
+
+extern "C" bkid_host_bgzf *bkid_host_bgzf_parse(const uint8_t *buf, const bkid_bgzf_block *blocks, int64_t n_blocks, int *need_more, char *err, int errlen)
+{
+  bkid_host_bgzf *h = new bkid_host_bgzf();
+  std::string msg;
+  int r = bam_header_parse(h, buf, blocks, n_blocks, false, msg);
+  if (need_more) *need_more = r == 0;
+  if (r != 1) { if (r < 0) set_err(err, errlen, msg); delete h; return nullptr; }
+  return h;
+}
 
 extern "C" bkid_host_bgzf *bkid_host_bgzf_open(const char *path, char *err, int errlen)
 {
@@ -352,69 +461,14 @@ extern "C" bkid_host_bgzf *bkid_host_bgzf_open(const char *path, char *err, int 
   close(fd);
   if (file == MAP_FAILED) { set_err(err, errlen, "mmap failed"); return nullptr; }
   bkid_host_bgzf *h = new bkid_host_bgzf();
-  h->file = file; h->fsz = fsz;
-  auto bail = [&](const char *msg) -> bkid_host_bgzf * { set_err(err, errlen, msg); munmap((void *)file, fsz); delete h; return nullptr; };
-  size_t off = 0;
-  while (off + 18 <= fsz) {
-    const uint8_t *p = file + off;
-    if (p[0] != 0x1f || p[1] != 0x8b) return bail("not a BGZF file");
-    uint16_t xlen = rd16(p + 10);
-    uint32_t bsize = 0;
-    if (off + 12 + xlen > fsz) return bail("corrupt BGZF block");
-    for (uint32_t x = 0; x + 4 <= xlen;) {        // every subfield must lie inside XLEN
-      const uint8_t *q = p + 12 + x;
-      uint16_t slen = rd16(q + 2);
-      if (x + 4 + (uint32_t)slen > xlen) break;
-      if (q[0] == 'B' && q[1] == 'C' && slen == 2) bsize = (uint32_t)rd16(q + 4) + 1;
-      x += 4 + slen;
-    }
-    if (!bsize || off + bsize > fsz || bsize < 12u + xlen + 8u) return bail("corrupt BGZF block");
-    bkid_bgzf_block b;
-    b.payload_off = off + 12 + xlen; b.payload_len = bsize - 12 - xlen - 8; b.usize = rd32(p + bsize - 4);
-    h->blocks.push_back(b);
-    h->usize += b.usize;
-    off += bsize;
-  }
-  if (off != fsz) return bail("trailing bytes after the last BGZF block");
-  // BAM header: inflate leading blocks until it is complete
-  std::vector<uint8_t> u;
-  size_t nb = 0;
-  auto need = [&](size_t bytes) -> bool {
-    while (u.size() < bytes && nb < h->blocks.size()) {
-      const bkid_bgzf_block &b = h->blocks[nb++];
-      size_t o = u.size();
-      u.resize(o + b.usize);
-      if (b.usize) {
-        z_stream zs; memset(&zs, 0, sizeof zs);
-        if (inflateInit2(&zs, -15) != Z_OK) return false;
-        zs.next_in = const_cast<uint8_t *>(file + b.payload_off); zs.avail_in = b.payload_len;
-        zs.next_out = u.data() + o; zs.avail_out = b.usize;
-        int r = inflate(&zs, Z_FINISH);
-        inflateEnd(&zs);
-        if (r != Z_STREAM_END || zs.total_out != b.usize) return false;
-      }
-    }
-    return u.size() >= bytes;
-  };
-  if (!need(12) || memcmp(u.data(), "BAM\1", 4) != 0) return bail("not a BAM file");
-  size_t o = 4;
-  uint32_t l_text = rd32(u.data() + o); o += 4;
-  if (!need(o + l_text + 4)) return bail("truncated BAM header");
-  o += l_text;
-  uint32_t n_ref = rd32(u.data() + o); o += 4;
-  for (uint32_t i = 0; i < n_ref; ++i) {
-    if (!need(o + 4)) return bail("truncated BAM header");
-    uint32_t l_name = rd32(u.data() + o); o += 4;
-    if (!need(o + l_name + 4)) return bail("truncated BAM header");
-    h->names.emplace_back((const char *)(u.data() + o)); o += l_name;
-    h->target_len.push_back(rd32(u.data() + o)); o += 4;
-  }
-  h->first_record = o;
-  if (need(o + 36)) h->first_l_qseq = (int32_t)rd32(u.data() + o + 20);
-  for (auto &s : h->names) h->name_ptrs.push_back(s.c_str());
-  h->hdr.n_targets = (int32_t)h->names.size();
-  h->hdr.target_len = h->target_len.data();
-  h->hdr.target_name = h->name_ptrs.data();
+  h->file = file; h->fsz = fsz; h->mapped = true;
+  auto bail = [&](const std::string &msg) -> bkid_host_bgzf * { set_err(err, errlen, msg); munmap((void *)file, fsz); delete h; return nullptr; };
+  std::string msg;
+  int64_t used = bgzf_walk(file, fsz, h->blocks, msg);
+  if (used < 0) return bail(msg);
+  if ((uint64_t)used != fsz) return bail(fsz - (uint64_t)used < 18 ? "trailing bytes after the last BGZF block" : "corrupt BGZF block");
+  for (const bkid_bgzf_block &b : h->blocks) h->usize += b.usize;
+  if (bam_header_parse(h, file, h->blocks.data(), (int64_t)h->blocks.size(), true, msg) != 1) return bail(msg);
   return h;
 }
 extern "C" const bkid_header *bkid_host_bgzf_header(const bkid_host_bgzf *h) { return &h->hdr; }
@@ -425,7 +479,12 @@ extern "C" int64_t bkid_host_bgzf_n_blocks(const bkid_host_bgzf *h) { return (in
 extern "C" uint64_t bkid_host_bgzf_first_record(const bkid_host_bgzf *h) { return h->first_record; }
 extern "C" uint64_t bkid_host_bgzf_usize(const bkid_host_bgzf *h) { return h->usize; }
 extern "C" int32_t bkid_host_bgzf_first_l_qseq(const bkid_host_bgzf *h) { return h->first_l_qseq; }
-extern "C" void bkid_host_bgzf_close(bkid_host_bgzf *h) { if (!h) return; munmap((void *)h->file, h->fsz); delete h; }
+extern "C" void bkid_host_bgzf_close(bkid_host_bgzf *h)
+{
+  if (!h) return;
+  if (h->mapped) munmap((void *)h->file, h->fsz);
+  delete h;
+}
 
 // ---- host half of the SAM path (bkid_push_sam): the @SQ lines of the header become the target table ----------
 struct bkid_host_sam {

@@ -31,6 +31,19 @@ uint64_t bkid_host_bgzf_usize(const bkid_host_bgzf *h);                 /* total
 int32_t bkid_host_bgzf_first_l_qseq(const bkid_host_bgzf *h);           /* read length of the first record (driver's _params.txt), -1 if none */
 void bkid_host_bgzf_close(bkid_host_bgzf *h);
 
+/* Host half of the stream path (bkid_push_bgzf_stream), for a BAM whose bytes arrive in order (a pipe):
+ * bkid_host_bgzf_walk  walks the whole BGZF blocks at the front of buf[0, len) into out[0, *n_blocks) (payload_off relative
+ *                      to buf; at most `cap` blocks, len / 28 + 1 always suffices) and returns the bytes they span.  An
+ *                      incomplete trailing block is not consumed: it is completed by the bytes that follow.  Returns -1
+ *                      and fills `err` when a block header is not BGZF (gzip magic, FEXTRA, BC subfield, BSIZE), which
+ *                      includes a plain gzip stream.  bkid_host_bgzf_open walks a file with the same code.
+ * bkid_host_bgzf_parse parses the BAM header from the leading blocks of such a prefix (zlib on just enough of them).
+ *                      NULL with *need_more = 1: the blocks end before the header does; NULL with *need_more = 0: not a
+ *                      BAM (err).  Otherwise the header and first_record; data / size / blocks / usize of the result are
+ *                      empty (the caller keeps the bytes), first_l_qseq is -1 unless the first record is in the prefix. */
+int64_t bkid_host_bgzf_walk(const uint8_t *buf, uint64_t len, bkid_bgzf_block *out, int64_t cap, int64_t *n_blocks, char *err, int errlen);
+bkid_host_bgzf *bkid_host_bgzf_parse(const uint8_t *buf, const bkid_bgzf_block *blocks, int64_t n_blocks, int *need_more, char *err, int errlen);
+
 /* Host half of the SAM path (bkid_push_sam): the header's @SQ SN:/LN: lines become the target table in @SQ order
  * (other header lines are ignored; a duplicate SN, an @SQ without SN, or a missing or non-numeric LN is an error).
  * The alignment lines start at first_record, on file line first_line (1-based).  A file without header lines is valid

@@ -17,20 +17,29 @@
 //   * -i may name SAM text instead of a BAM (a file whose first line is a header line or an alignment line of 11 or more
 //     tab-separated fields), or be - to read SAM from stdin: the lines are parsed on the device (bkid_push_sam), and no
 //     .bai is required.  A BAM (first bytes 1f 8b) takes the BAM path unchanged.  With -gpu a,b,... every rank parses
-//     the newline-aligned byte range of a coordinate-sorted SAM file that falls to it; stdin needs one GPU.
+//     the newline-aligned byte range of a coordinate-sorted SAM file that falls to it; stdin needs one GPU;
+//   * -i - (stdin) and any -i path that is not a regular file (a FIFO, /dev/fd/N of a pipe or a process substitution,
+//     /dev/stdin on a pipe) are read as a stream, so `samtools markdup -u in.bam - | BreakID -i -` needs no file on disk.
+//     The first bytes decide the format: 1f 8b is a BAM, decoded on the device piece by piece as it arrives while a reader
+//     thread fills the next piece (bkid_push_bgzf_stream); anything else is SAM text (bkid_push_sam).  One GPU, no .bai.
 // Host work: BAM / SAM header parsing (bam_reader.cc), .nib loading, refGene annotation, the final unstable sort
 // by N_DRP and file writing.  Everything between decode and the cluster records runs on the GPU.
+#include <errno.h>
+#include <fcntl.h>
 #include <getopt.h>
 #include <sys/stat.h>
+#include <unistd.h>
 
 #include <algorithm>
 #include <chrono>
 #include <cmath>
+#include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
 #include <iostream>
+#include <mutex>
 #include <set>
 #include <string>
 #include <thread>
@@ -45,7 +54,7 @@ static const char *kHelp =
     " Usage: \n \t BreakID -i input.bam -o prefix -n nib_folder <options> \n\n "
     "     DESCRIPTION\n "
     "     \t -h -? -help \t help\n "
-    "     \t -i*        \t input bam-file, or SAM text (a file, or - for stdin)\n "
+    "     \t -i*        \t input BAM or SAM text: a file, a pipe / FIFO, or - for stdin\n "
     "     \t -o*        \t output file (prefix only)\n "
     "     \t -n*        \t folder name to nib files\n "
     "     \t -q         \t encompassing reads quality thresholds  [20]\n"
@@ -84,6 +93,46 @@ static int sniff_input(const std::string &path)
   std::string first = b.substr(0, b.find('\n'));
   return std::count(first.begin(), first.end(), '\t') >= 10 ? 1 : -1;
 }
+
+// A stream input (stdin, a FIFO, a pipe): a reader thread appends what arrives to `buf` while the caller works on what
+// it took before.  The reader pauses while `buf` holds `high` bytes (or what the caller waits for), so memory stays bounded.
+struct StreamReader {
+  int fd = -1;
+  size_t high = 0, want = 0;
+  std::vector<uint8_t> buf;                            // bytes read and not yet taken
+  bool eof = false;
+  int err = 0;                                         // errno of a failed read
+  std::mutex m;
+  std::condition_variable cv;
+  std::thread th;
+  void start()
+  {
+    th = std::thread([this] {
+      std::vector<uint8_t> chunk((size_t)4 << 20);
+      for (;;) {
+        ssize_t n = read(fd, chunk.data(), chunk.size());
+        if (n < 0 && errno == EINTR) continue;
+        std::unique_lock<std::mutex> l(m);
+        if (n <= 0) { eof = true; err = n < 0 ? errno : 0; cv.notify_all(); return; }
+        cv.wait(l, [&] { return buf.size() < std::max(high, want); });
+        buf.insert(buf.end(), chunk.data(), chunk.data() + n);
+        cv.notify_all();
+      }
+    });
+  }
+  // wait until at least `bytes` are buffered or the stream has ended, then run f(buf, eof) under the lock
+  template <class F> void take(size_t bytes, F f)
+  {
+    std::unique_lock<std::mutex> l(m);
+    want = bytes;
+    cv.notify_all();
+    cv.wait(l, [&] { return buf.size() >= bytes || eof; });
+    f(buf, eof);
+    want = 0;
+    cv.notify_all();
+  }
+  void join() { if (th.joinable()) th.join(); }
+};
 
 static bool cmp_cluster(const CallRow &a, const CallRow &b) { return a.c.n_discordant_pair > b.c.n_discordant_pair; }   // reference src/BreakID.h:185-188
 
@@ -244,21 +293,42 @@ int main(int argc, char *argv[])
   bkid_host_sam *sam = nullptr;
   const bkid_header *hdr = nullptr;
   const bool from_stdin = inp == "-";
-  const bool is_sam = from_stdin || sniff_input(inp) == 1;
-  std::vector<uint8_t> sbuf;                           // stdin: the text read so far and not yet pushed
-  size_t spos = 0;                                     // stdin: start of the unpushed text in sbuf
+  struct stat ist;
+  const bool stream = from_stdin || (stat(inp.c_str(), &ist) == 0 && (S_ISFIFO(ist.st_mode) || S_ISCHR(ist.st_mode) || S_ISSOCK(ist.st_mode)));
+  if (stream && gpus.size() > 1) {
+    std::cerr << "Error: " << (from_stdin ? std::string("stdin") : "a stream (" + inp + ")") << " needs one GPU; give a file to use several (-gpu " << gpus.size() << " devices)\n";
+    exit(1);
+  }
+  if (stream && host_decode) { std::cerr << "Error: host decode reads a BAM file (unset BKID_HOST_DECODE to read a stream)\n"; exit(1); }
+  const int sfd = !stream ? -1 : from_stdin ? 0 : open(inp.c_str(), O_RDONLY);
+  if (stream && sfd < 0) { std::cerr << "Error: can not open bam-file: " << inp << std::endl; exit(1); }
+  std::vector<uint8_t> sbuf;                           // stream: the bytes read so far and not yet pushed
+  size_t spos = 0;                                     // stream: start of the unpushed text in sbuf
   bool seof = false;
   const size_t PIECE = (size_t)256 << 20;
-  auto sfill = [&]() {
-    size_t o = sbuf.size();
-    sbuf.resize(o + PIECE);
-    size_t n = fread(sbuf.data() + o, 1, PIECE, stdin);
-    sbuf.resize(o + n);
-    if (n == 0) seof = true;
+  auto sread = [&](size_t max) {                       // append up to `max` bytes of the stream to sbuf (less only at its end)
+    size_t o = sbuf.size(), got = 0;
+    sbuf.resize(o + max);
+    while (got < max) {
+      ssize_t n = read(sfd, sbuf.data() + o + got, max - got);
+      if (n < 0 && errno == EINTR) continue;
+      if (n <= 0) break;
+      got += (size_t)n;
+    }
+    sbuf.resize(o + got);
+    if (got < max) seof = true;
   };
+  auto sfill = [&]() { sread(PIECE); };
+  if (stream) sread(2);                                // the first bytes decide the format
+  const bool bam_stream = stream && sbuf.size() >= 2 && sbuf[0] == 0x1f && sbuf[1] == 0x8b;
+  const bool sam_stream = stream && !bam_stream;
+  const bool is_sam = sam_stream || (!stream && sniff_input(inp) == 1);
   if (is_sam && host_decode) { std::cerr << "Error: host decode reads BAM only (unset BKID_HOST_DECODE for SAM input)\n"; exit(1); }
-  if (from_stdin && gpus.size() > 1) { std::cerr << "Error: SAM from stdin needs one GPU; give a SAM file to use several (-gpu " << gpus.size() << " devices)\n"; exit(1); }
-  if (from_stdin) {
+  // BAM stream: pieces of at least this much go to the device (BKID_STREAM_PIECE_KB sets it, e.g. to test many pieces)
+  size_t piece_bytes = (size_t)256 << 20;
+  if (const char *e = getenv("BKID_STREAM_PIECE_KB")) if (atol(e) >= 64) piece_bytes = (size_t)atol(e) << 10;
+  StreamReader reader;
+  if (sam_stream) {
     for (;;) {                                         // the header lines come first
       if (spos >= sbuf.size()) { if (seof) break; sfill(); continue; }
       if (sbuf[spos] != '@') break;
@@ -267,8 +337,33 @@ int main(int argc, char *argv[])
       spos = (size_t)((const uint8_t *)nl - sbuf.data()) + 1;
     }
     sam = bkid_host_sam_parse(sbuf.data(), spos, err, sizeof err);
-    if (!sam) { std::cerr << "Error: can not read sam header from stdin: " << err << std::endl; exit(1); }
+    if (!sam) { std::cerr << "Error: can not read sam header from " << (from_stdin ? std::string("stdin") : inp) << ": " << err << std::endl; exit(1); }
     hdr = bkid_host_sam_header(sam);
+  } else if (bam_stream) {
+    // the BAM header comes first: wait for the blocks that hold it (nothing is consumed here)
+    reader.fd = sfd;
+    reader.high = 4 * piece_bytes;
+    reader.buf.swap(sbuf);
+    reader.start();
+    std::string msg;
+    for (size_t seen = 0;;) {
+      bool more = false;
+      reader.take(seen + 1, [&](std::vector<uint8_t> &b, bool eof) {
+        seen = b.size();
+        std::vector<bkid_bgzf_block> tb(b.size() / 28 + 1);
+        int64_t nb = 0;
+        if (bkid_host_bgzf_walk(b.data(), b.size(), tb.data(), (int64_t)tb.size(), &nb, err, sizeof err) < 0) { msg = err; return; }
+        int need_more = 0;
+        bgzf = bkid_host_bgzf_parse(b.data(), tb.data(), nb, &need_more, err, sizeof err);
+        if (bgzf) return;
+        if (!need_more) msg = err;
+        else if (eof) msg = reader.err ? std::string("read error: ") + strerror(reader.err) : std::string("the stream ends inside the BAM header");
+        else more = true;
+      });
+      if (!more) break;
+    }
+    if (!bgzf) { std::cerr << "Error: can not read bam-file: " << inp << " (" << msg << ")" << std::endl; exit(1); }
+    hdr = bkid_host_bgzf_header(bgzf);
   } else if (is_sam) {
     sam = bkid_host_sam_open(inp.c_str(), err, sizeof err);
     if (!sam) { std::cerr << "Error: can not open sam-file: " << inp << " (" << err << ")" << std::endl; exit(1); }
@@ -410,6 +505,7 @@ int main(int argc, char *argv[])
   double t_push0 = now_s();
   bkid_decode_stats dst;
   memset(&dst, 0, sizeof dst);
+  int64_t n_pieces = 0;
   if (host_decode) {
     if (bkid_push_batch(ctx, bkid_host_bam_batch_narrow(bam))) die("push_batch");
   } else if (sam) {
@@ -426,7 +522,7 @@ int main(int argc, char *argv[])
       return nrec;
     };
     int64_t line = bkid_host_sam_first_line(sam);
-    if (!from_stdin) {
+    if (!sam_stream) {
       const uint64_t f0 = bkid_host_sam_first_record(sam);
       push(bkid_host_sam_data(sam) + f0, bkid_host_sam_size(sam) - f0, line);
     } else {
@@ -444,6 +540,37 @@ int main(int argc, char *argv[])
         sfill();
       }
     }
+  } else if (bam_stream) {
+    // each push takes every whole block read so far once the previous push has returned and `piece_bytes` are buffered
+    // (or the stream has ended); the partial block at the end goes back in front of what the reader appends next
+    auto bad = [&](const std::string &why) { std::cerr << "Error: can not read bam-file: " << inp << " (" << why << ")" << std::endl; exit(1); };
+    if (bkid_bgzf_stream_begin(ctx, bkid_host_bgzf_first_record(bgzf))) bad(bkid_last_error(ctx));
+    std::vector<uint8_t> piece;
+    std::vector<bkid_bgzf_block> tb;
+    for (bool last = false; !last;) {
+      int64_t nb = 0, used = 0;
+      int rerr = 0;
+      reader.take(piece_bytes, [&](std::vector<uint8_t> &b, bool eof) {
+        last = eof; rerr = reader.err;
+        tb.resize(b.size() / 28 + 1);
+        used = bkid_host_bgzf_walk(b.data(), b.size(), tb.data(), (int64_t)tb.size(), &nb, err, sizeof err);
+        if (used < 0) return;
+        piece.assign(b.begin() + used, b.end());
+        std::swap(piece, b);                             // piece: the whole blocks (and the tail), b: the tail
+      });
+      if (used < 0) bad(err);
+      if (rerr) bad(std::string("read error: ") + strerror(rerr));
+      if (last && (size_t)used != piece.size()) bad("the stream ends inside a BGZF block");
+      int64_t nrec = 0;
+      if (nb) {
+        if (bkid_push_bgzf_stream(ctx, piece.data(), (uint64_t)used, tb.data(), nb, &nrec)) bad(bkid_last_error(ctx));
+        ++n_pieces;
+      }
+    }
+    int64_t nrec = 0;
+    if (bkid_bgzf_stream_end(ctx, &nrec)) bad(bkid_last_error(ctx));
+    reader.join();
+    bkid_get_decode_stats(ctx, &dst);
   } else {
     int64_t nrec = 0;
     if (bkid_push_bgzf(ctx, bkid_host_bgzf_data(bgzf), bkid_host_bgzf_size(bgzf), bkid_host_bgzf_blocks(bgzf), bkid_host_bgzf_n_blocks(bgzf), bkid_host_bgzf_first_record(bgzf), &nrec)) {
@@ -479,7 +606,7 @@ int main(int argc, char *argv[])
   std::vector<bkid_cluster_rec> cl;
   double t_bp = 0;
   if (tm.n_clustered > 0) {
-    if (!sort && !sam && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
+    if (!sort && !sam && !stream && !exists(inp + ".bai") && !exists(inp.substr(0, inp.size() > 4 ? inp.size() - 4 : 0) + ".bai")) {
       std::cerr << "Error: please index bam-file first:\t" << inp << std::endl;                     // src/BreakID.cc:412-416
       exit(1);
     }
@@ -500,7 +627,7 @@ int main(int argc, char *argv[])
     cl.resize((size_t)n);
   }
   bkid_get_timings(ctx, &tm);
-  finish_and_write(inp, out, refgene, names, cl, filter, !sort && !sam, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
+  finish_and_write(inp, out, refgene, names, cl, filter, !sort && !sam && !stream, qual, dist, tm.n_clustered > 0, t_start, n_pairs, tm.n_masked, tm.n_clustered, n_clusters, t_scan, t_cluster, t_bp,
                    [&](std::ofstream &j) {
                      if (sam)
                        j << "decoder\tsam\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ntext_bytes\t" << dst.uncompressed_bytes << "\nlines_ms\t" << dst.boundaries_ms << "\nparse_ms\t" << dst.extract_ms
@@ -508,6 +635,7 @@ int main(int argc, char *argv[])
                      else
                        j << "decoder\t" << (host_decode ? "host" : "device") << "\nopen_s\t" << t_decode << "\npush_s\t" << t_push << "\ninflate_ms\t" << dst.inflate_ms << "\nboundaries_ms\t" << dst.boundaries_ms
                          << "\nextract_ms\t" << dst.extract_ms << "\ncompressed_bytes\t" << dst.compressed_bytes << "\nuncompressed_bytes\t" << dst.uncompressed_bytes;
+                     if (bam_stream) j << "\nstream\t1\npieces\t" << n_pieces;
                      j << "\nrecords\t" << tm.n_records << "\nh2d_ms\t" << tm.h2d << "\nclassify_ms\t" << tm.classify << "\ninsert_stats_ms\t" << tm.insert_stats
                        << "\njoin_ms\t" << tm.join << "\nbucket_sort_ms\t" << tm.bucket_sort << "\nmask_ms\t" << tm.mask << "\ncluster_ms\t" << tm.cluster << "\nsummarize_ms\t" << tm.summarize
                        << "\nevidence_ms\t" << tm.evidence << "\nrefine_ms\t" << tm.refine << "\n";

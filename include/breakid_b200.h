@@ -228,6 +228,28 @@ int bkid_push_bgzf(bkid_ctx *ctx, const uint8_t *file, uint64_t file_size, const
 int bkid_push_bgzf_range(bkid_ctx *ctx, const uint8_t *file, uint64_t file_size, const bkid_bgzf_block *blocks, int64_t n_blocks,
                          uint64_t first_record_uoffset, int64_t first_block, int64_t end_block, int64_t *n_records,
                          uint64_t *first_record_uoff, uint64_t *next_record_uoff);
+/* Extension (the reference opens a file): decode a BAM that arrives as a byte stream, e.g. on a pipe, one piece at a time.
+ * For any BAM byte stream cut into pieces in any way, begin + one push per piece + end leaves the context in exactly the
+ * state bkid_push_bgzf leaves for the same bytes held as a file (every bkid_fetch_column column, the counts, have_seq).
+ *   bkid_bgzf_stream_begin  opens a session; first_record_uoffset = size of the BAM header (bam_reader.h:
+ *                           bkid_host_bgzf_parse parses it from the first bytes of the stream).
+ *   bkid_push_bgzf_stream   `piece` holds the next whole BGZF blocks of the stream, in order, the first piece starting at
+ *                           byte 0; `blocks` is their table with payload_off relative to `piece` (bkid_host_bgzf_walk),
+ *                           validated against piece_size.  Pinned pieces are copied from directly, pageable ones through
+ *                           the library's pinned staging, which a session keeps.  The records that complete in the piece
+ *                           are appended (*n_records); the partial record at its end (device memory, up to 64 MiB) and
+ *                           the rest of a BAM header spread over several pieces carry over to the next push.  Column
+ *                           capacity grows geometrically (the total is unknown; bkid_reserve still applies).
+ *   bkid_bgzf_stream_end    closes the session; *n_records = records of the whole session.
+ * Errors: a deflate error, CRC32 mismatch or wrong ISIZE (naming the block by its index in the stream), a corrupt record, a
+ * record over 64 MiB and, at end, a record still carried return BKID_ERR_IO with bkid_push_bgzf's message.  Any error ends
+ * the session and the context then holds exactly what it held at begin.  BKID_ERR_ARG: begin on a context holding borrowed
+ * device columns, begin twice, push or end without begin, and any other push, sort or stage call while a session is open.
+ * bkid_reset closes a session.  bkid_get_decode_stats accumulates over the session. */
+int bkid_bgzf_stream_begin(bkid_ctx *ctx, uint64_t first_record_uoffset);
+int bkid_push_bgzf_stream(bkid_ctx *ctx, const uint8_t *piece, uint64_t piece_size, const bkid_bgzf_block *blocks, int64_t n_blocks,
+                          int64_t *n_records);
+int bkid_bgzf_stream_end(bkid_ctx *ctx, int64_t *n_records);
 int bkid_get_decode_stats(bkid_ctx *ctx, bkid_decode_stats *stats);
 /* Extension (the reference reads BAM only): append the records of SAM alignment text, parsed on the device.
  * `text` holds alignment lines only (no header), in host memory (pinned memory is copied from directly, pageable memory
